@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — step-2 K=60 graph build throughput (Gbases/s) on N B200s; see DESIGN.md §Measurement.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--genome-mbp G] [--coverage C] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--genome-mbp G] [--coverage C] [--impl reference] [--dump-outputs DIR]
 
 One step = one whole pass of step 2 (count -> adjacency -> unipaths -> HBV -> read pathing) over one synthetic read set.
 `value` = bases / device time with the read stores already resident in HBM; `e2e` = the same through w2rap_step2_run()
@@ -198,6 +198,31 @@ def digest_reference(key):
     return None
 
 
+DUMP_ARRAYS = ("hist", "edge_off", "edge_len", "edge_bases", "edge_vertices", "fwd_xlat", "rev_xlat", "involution",
+               "path_offset", "path_off", "path_edges", "place_off", "place_edges")
+DUMP_COUNTS = ("n_reads", "n_bases", "n_kmer_instances", "n_distinct", "n_solid", "n_edges", "n_edge_bases", "n_vertices", "n_hbv_edges",
+               "n_paths", "n_path_edges", "n_pathed", "n_multipathed", "n_places_kept", "n_places")
+DUMP_CAP = 1 << 19          # elements kept per array: the 13 arrays and the counters stay under 64 MB in float64
+
+
+def dump_outputs(d, out_dir):
+    """Writes the w2rap_graph `d` (a T.graph_to_dict) as out_dir/<field>.npy in float64, which holds every value exactly (all are
+    below 2^53).  An array longer than DUMP_CAP is replaced by its elements at DUMP_CAP sorted positions drawn with a fixed seed, so
+    two builds that agree on its length sample the same positions.  An array the step did not fill (the places without --places) is
+    not written.  counts.npy holds the counters in DUMP_COUNTS order, then the graph and path digests as 32-bit halves (high, low)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name in DUMP_ARRAYS:
+        a = np.asarray(d[name]).reshape(-1)
+        if a.size == 0:
+            continue
+        if a.size > DUMP_CAP:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_CAP, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+    digests = [x for k in ("digest_graph", "digest_paths") for x in (d[k] >> 32, d[k] & 0xffffffff)]
+    np.save(os.path.join(out_dir, "counts.npy"), np.array([d[k] for k in DUMP_COUNTS] + digests, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -213,7 +238,15 @@ def main():
     ap.add_argument("--places", type=int, default=0, help="also build step 3's places for this large K inside the timed step (SURVEY N1; off by default: not part of the metric)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer (e2e) legs: for workloads whose reads do not fit pinned host memory")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the graph and paths the last timed step returned as DIR/<name>.npy (float64; arrays longer than %d elements as a "
+                         "fixed seeded sample of that many; the places only with --places; in a sharded run rank 0's: the graph and the paths "
+                         "of its reads)" % DUMP_CAP)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the B200 path returns; the reference arm has no such output")
     preset = {"c1": (4.6, 100, 0), "c2": (135.0, 60, 0), "c3": (1000.0, 60, 100), "custom": (135.0, 60, 0)}[args.config]
     if args.genome_mbp is None:
         args.genome_mbp = preset[0]
@@ -279,7 +312,9 @@ def main():
     def timings_of(g):
         return {n: (list(getattr(g.timings, n)) if n == "kernel_ms" else getattr(g.timings, n)) for n, _ in T.Timings._fields_}
 
-    def step_resident():
+    kept = {}
+
+    def step_resident(keep=False):
         g = T.Graph()
         rc = lib.w2rap_step2_run_sharded_resident(h, C.byref(p), comm, C.byref(g), err, 1024) if world > 1 else lib.w2rap_step2_run_resident(h, C.byref(p), C.byref(g), err, 1024)
         if rc:
@@ -287,6 +322,8 @@ def main():
         t = timings_of(g)
         t["n_places_kept"], t["n_places"] = int(g.n_places_kept), int(g.n_places)
         info = (int(g.n_kmer_instances), int(g.n_distinct), int(g.n_solid), int(g.n_edges), int(g.n_edge_bases), int(g.n_pathed), int(g.n_path_edges), int(g.digest_graph), int(g.digest_paths))
+        if keep:
+            kept["graph"] = T.graph_to_dict(g)      # host copy after the step's own timings were taken
         lib.w2rap_step2_free(C.byref(g))
         return t, info
 
@@ -312,13 +349,15 @@ def main():
     th.start()
     barrier()
     tt, info = [], None
-    for _ in range(args.steps):
-        t, info2 = step_resident()
+    for i in range(args.steps):
+        t, info2 = step_resident(keep=args.dump_outputs is not None and rank == 0 and i == args.steps - 1)
         if info is not None and info2 != info:
             raise SystemExit("non-deterministic result between steps: %r vs %r" % (info, info2))
         info = info2
         tt.append(t)
     barrier()
+    if kept:
+        dump_outputs(kept.pop("graph"), args.dump_outputs)
     dev_ms = median([t["total_ms"] - t["d2h_ms"] for t in tt])      # device time, results left on the device side of the copy
     full_ms = median([t["total_ms"] for t in tt])
     # end to end through the host-buffer entry point: pinned host buffers, then pageable ones
@@ -400,8 +439,9 @@ def main():
     if not args.no_cpu_baseline and world == 1:
         try:
             same = same_input_comparison(args, lib, local)
+            arm = "oracle/_ref/w2rap-contigger --from_step 2 --to_step 2, TIME buildReadQGraph+FixPaths" if same["cpu_kind"] == "reference" else "oracle/step2_oracle.c"
             cpu = {"value": same["cpu_gbases_per_s"], "unit": "Gbases/s", "cores": same["cpu_cores"], "kind": same["cpu_kind"],
-                   "sample": same["sample"] + "; oracle/_ref/w2rap-contigger --from_step 2 --to_step 2, TIME buildReadQGraph+FixPaths (bounded sample: the ratio to `value` is indicative; `same_input` holds the like-for-like one)"}
+                   "sample": same["sample"] + "; " + arm + " (bounded sample: the ratio to `value` is indicative; `same_input` holds the like-for-like one)"}
         except Exception as e:   # the baseline is reported, never required
             cpu = {"value": None, "unit": "Gbases/s", "cores": os.cpu_count(), "kind": "unavailable", "sample": repr(e)[:200]}
     wkey = "genome%.1fMbp_cov%d_len%d_het%d_seed1000" % (args.genome_mbp, args.coverage, args.read_len, args.het)

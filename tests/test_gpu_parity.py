@@ -257,12 +257,15 @@ def test_size_independent_properties_at_scale(T):
 def test_reference_binary_with_dropin_translation_unit(T, tmp_path):
     """The reference's own main() with only src/paths/long/BuildReadQGraph.cc swapped for host/BuildReadQGraph_b200.cc
     (oracle/_ref/w2rap-contigger-b200, linked by `make -C oracle dropin`): --from_step 2 --to_step 2 must write the same
-    step-2 files as the unmodified reference did for tests/golden (modulo its racy edge numbering)."""
+    step-2 files as the unmodified reference did for tests/golden (modulo its racy edge numbering).  It links the reference's own
+    object files, so no stored output can stand in for it: it skips unless the reference was built from its sources (W2RAP_REFERENCE
+    at build time).  The same golden files are compared with the library itself in test_golden_reference_outputs and
+    test_standalone_step2_binary, which always run."""
     import shutil
     import subprocess
     exe = os.path.join(os.path.dirname(T.REF_BIN), "w2rap-contigger-b200")
     if not os.path.exists(exe):
-        pytest.skip("drop-in binary not built (needs /root/reference at build time)")
+        pytest.skip("drop-in binary not built (needs the reference's sources: W2RAP_REFERENCE=<checkout> at build time)")
     for case in ("circ", "rich"):
         d = str(tmp_path / case)
         os.makedirs(d)
@@ -302,9 +305,10 @@ def test_standalone_step2_binary(T, tmp_path):
 def test_config1_against_the_reference_binary(T, tmp_path):
     """BASELINE.json configs[0] at full size — E. coli-sized 4.6 Mbp genome, 2x250 PE at 100x, 1.84 M reads — through the UNMODIFIED
     reference binary (oracle/_ref/w2rap-contigger, all host threads) and through the B200 path, same reads: histogram, edge set,
-    vertices and every read path must agree (modulo the reference's racy edge numbering and its extension ties)."""
+    vertices and every read path must agree (modulo the reference's racy edge numbering and its extension ties).  It runs the
+    reference itself and skips without it; test_config1_against_the_oracle runs the same reads against the oracle everywhere."""
     if not os.path.exists(T.REF_BIN):
-        pytest.skip("oracle/_ref/w2rap-contigger not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/w2rap-contigger not built (needs the reference's sources: W2RAP_REFERENCE=<checkout> at build time)")
     lib = T.product_lib()
     err = C.create_string_buffer(512)
     sp = T.SynthParams(4_600_000, 250, 100, 11, 0, 0, 0, 0)
@@ -327,6 +331,33 @@ def test_config1_against_the_reference_binary(T, tmp_path):
     rep = T.compare_with_reference_fast(got, T.graph_from_reference_files(d))
     assert rep["edge_set_equal"] and rep["hist_equal"] and rep["vertices_equal"], {k: v for k, v in rep.items() if k != "path_mismatches"}
     assert rep["path_mismatches"] == [] and rep["path_ties"] <= 50, (rep["path_ties"], rep["path_mismatches"][:10])
+    assert got["n_pathed"] > 0.97 * got["n_reads"]
+
+
+def test_config1_against_the_oracle(T):
+    """BASELINE.json configs[0] at full size (the reads of test_config1_against_the_reference_binary: 4.6 Mbp, 100x, 1.84 M reads,
+    seed 11) through the B200 path and through the oracle, whose restatement is pinned on the reference's own files
+    (test_oracle_golden.py): every array bit for bit, at a size the other parity tests do not reach.  Runs without the reference."""
+    lib = T.product_lib()
+    err = C.create_string_buffer(512)
+    sp = T.SynthParams(4_600_000, 250, 100, 11, 0, 0, 0, 0)
+    h = C.c_void_p()
+    assert lib.w2rap_step2_synth(C.byref(sp), -1, C.byref(h), err, 512) == 0, err.value
+    r = T.Reads()
+    assert lib.w2rap_step2_download_reads(h, C.byref(r), err, 512) == 0, err.value
+    n = int(r.n_reads)
+    assert n == 1_840_000
+    boff, qoff = T._arr(r.base_off, n + 1, "<u8"), T._arr(r.qual_off, n + 1, "<u8")
+    rs = T.ReadSet(T._arr(r.bases, int(boff[-1]), "u1"), boff, T._arr(r.len, n, "<u4"), T._arr(r.quals, int(qoff[-1]), "u1"), qoff)
+    lib.w2rap_step2_free_host_reads(C.byref(r))
+    g = T.Graph()
+    p = T.default_params(apply_fixpaths=1, dump_kmers=1)
+    assert lib.w2rap_step2_run_resident(h, C.byref(p), C.byref(g), err, 512) == 0, err.value
+    got = T.graph_to_dict(g)
+    lib.w2rap_step2_free(C.byref(g))
+    lib.w2rap_step2_release(h)
+    want = T.run_oracle(rs, T.default_params(apply_fixpaths=1, dump_kmers=1))
+    T.assert_graph_equal(want, got, "config 1")
     assert got["n_pathed"] > 0.97 * got["n_reads"]
 
 

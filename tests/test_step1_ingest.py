@@ -142,8 +142,11 @@ def tricky_reads(seed, n_pairs):
 
 
 def test_against_the_reference_binary_on_fresh_fastq(T, s1, tmp_path):
+    """Runs the reference's own step 1, so it needs the reference built from its sources (W2RAP_REFERENCE at build time) and skips
+    without it; test_golden_step1_files_byte_for_byte (files the reference wrote) and test_stores_feed_step2_formats ('N' and lower
+    case on these kinds of reads) keep running."""
     if not os.path.exists(T.REF_BIN):
-        pytest.skip("oracle/_ref/w2rap-contigger not built")
+        pytest.skip("oracle/_ref/w2rap-contigger not built (needs the reference's sources: W2RAP_REFERENCE=<checkout> at build time)")
     seqs, quals = tricky_reads(5, 400)
     fq1, fq2 = write_fastq_pair(str(tmp_path), seqs, quals)
     ref = tmp_path / "ref"; ref.mkdir()
