@@ -446,10 +446,16 @@ struct Pipeline {
         if (bt.count) W2R_TIMED(W2RAP_KT_GOOD_LEN, W2R_LAUNCH(c, k_good_len, grid(bt.count, 128), 128, 0, dr.view(), bt.first, bt.count, prm.min_qual, good.p, cs_scal.p, cs_flags.p));
     }
 
+    static unsigned map_ctas() {
+        static const unsigned n = getenv("W2RAP_MAP_CTAS") ? (unsigned)atoi(getenv("W2RAP_MAP_CTAS")) : 6u;
+        return n;
+    }
+    // warps of the map launch over `count` reads that take a staging chunk: each ends the launch holding one partly used chunk
+    uint64_t map_chunk_warps(uint64_t count) const { return std::min<uint64_t>(count, (uint64_t)grid(count * 32, 256, map_ctas()) * 8); }
+
     // map: per read batch  quality floor -> counting launch -> scan -> store launch (all queued without a host round trip, so a
     // batch is mapped as soon as it has crossed PCIe).  Returns false if the record area was too small (need = exact size).
     bool map_records(const CountPlan& pl, CountBufs& cb, const std::vector<Batch>& batches, uint32_t pass, uint64_t* need) {
-        static const unsigned map_ctas = getenv("W2RAP_MAP_CTAS") ? (unsigned)atoi(getenv("W2RAP_MAP_CTAS")) : 6u;
         const ReadsView rv = dr.view();
         const uint64_t P = pl.P;
         cb.cursor.zero(); cb.part_count.zero(); cb.part_kcount.zero();
@@ -472,7 +478,7 @@ struct Pipeline {
             W2R_CUDA(cudaEventCreate(&ev[2 * bi])); W2R_CUDA(cudaEventCreate(&ev[2 * bi + 1]));
             W2R_CUDA(cudaEventRecord(ev[2 * bi], c.stream));
             W2R_LAUNCH(c, k_copy_scalar, 1, 1, 0, (const unsigned long long*)cb.tmp_cursor.p, cb.tmp_range.p + bi);
-            if (bt.count && pl.n_inst_local) W2R_TIMED(W2RAP_KT_MAP, W2R_LAUNCH(c, k_minimizer_map, grid(bt.count * 32, 256, map_ctas), 256, 0, rv, bt.first, bt.count, good.p, mp));
+            if (bt.count && pl.n_inst_local) W2R_TIMED(W2RAP_KT_MAP, W2R_LAUNCH(c, k_minimizer_map, grid(bt.count * 32, 256, map_ctas()), 256, 0, rv, bt.first, bt.count, good.p, mp));
             W2R_LAUNCH(c, k_copy_scalar, 1, 1, 0, (const unsigned long long*)cb.tmp_cursor.p, cb.tmp_range.p + bi + 1);
             exclusive_scan<uint32_t, uint64_t>(c, cb.part_count.p + bi * P, P, cb.part_base.p + bi * P, cb.batch_total.p + bi);
             W2R_LAUNCH(c, k_next_batch_off, 1, 1, 0, cb.batch_off.p + bi, cb.batch_total.p + bi);
@@ -722,8 +728,12 @@ struct Pipeline {
                 pl.npass *= 2; --attempt; continue;              // (more passes are not a failed attempt)
             }
             CountBufs cb;
-            // staging: the same records plus the unused ends of the chunks the warps reserve
-            const size_t stage_recs = local_recs + local_recs / 8 + (size_t)c.sm_count * 6 * 8 * MAP_CHUNK;
+            // staging: the same records plus the unused ends of the chunks the warps reserve, one per warp in every map launch (one
+            // launch per read batch)
+            uint64_t chunk_warps = 0;
+            if (world > 1) chunk_warps = map_chunk_warps(dr.n);
+            else for (const Batch& bt : batches) chunk_warps += map_chunk_warps(bt.count);
+            const size_t stage_recs = local_recs + local_recs / 8 + chunk_warps * MAP_CHUNK;
             cb.tmp_cursor.alloc(c, 1); cb.tmp_range.alloc(c, pl.nmap + 1);
             cb.part_count.alloc(c, pl.nmap * P); cb.part_kcount.alloc(c, pl.nmap * P); cb.cursor.alloc(c, pl.nmap * P);
             cb.part_base.alloc(c, pl.nmap * P); cb.batch_total.alloc(c, pl.nmap); cb.batch_ktotal.alloc(c, pl.nmap);
@@ -1699,10 +1709,26 @@ static void dev_alloc(DeviceReads* d, void** p, size_t bytes, cudaStream_t s, in
     }
     if (d->pooled) W2R_CUDA(cudaMallocAsync(p, bytes, s)); else W2R_CUDA(cudaMalloc(p, bytes));
 }
-// Validates the flattened store and starts its transfer.  With `batched`, the copy is issued as up to 8 read batches with an
-// event each and NOT waited for: the pipeline consumes batch b while batch b+1 is in flight.  Host buffers must stay valid until
-// the stream has drained (the entry points synchronise before returning).
+// W2RAP_UPLOAD_BATCHES=n (test hook): the host-buffer entry points split every non-empty read set into exactly n read batches, so
+// that the multi-run count (one record run per batch in every partition) can be checked on small read sets.  0 when unset, -1
+// when set to anything but 1..SMEM_MAX_BATCH.
+static int upload_batches_override() {
+    static const int n = [] {
+        const char* v = getenv("W2RAP_UPLOAD_BATCHES");
+        if (!v) return 0;
+        char* end = nullptr;
+        const long x = strtol(v, &end, 10);
+        return (end != v && *end == '\0' && x >= 1 && x <= (long)SMEM_MAX_BATCH) ? (int)x : -1;
+    }();
+    return n;
+}
+
+// Validates the flattened store and starts its transfer.  With `batched`, the copy is issued as read batches (8 from 2^20 reads on,
+// else 1, or as W2RAP_UPLOAD_BATCHES says) with an event each and NOT waited for: the pipeline consumes batch b while batch b+1 is
+// in flight.  Host buffers must stay valid until the stream has drained (the entry points synchronise before returning).
 static void upload(const w2rap_reads* in, int device, DeviceReads* d, cudaStream_t s, bool batched) {
+    const int forced_batches = batched ? upload_batches_override() : 0;
+    if (forced_batches < 0) W2R_FAIL(W2RAP_ERR_BAD_ARG, "W2RAP_UPLOAD_BATCHES must be an integer in 1..%u (the most record runs per partition the count handles)", SMEM_MAX_BATCH);
     d->device = device;
     d->n = in->n_reads;
     const uint64_t n = d->n;
@@ -1754,7 +1780,7 @@ static void upload(const w2rap_reads* in, int device, DeviceReads* d, cudaStream
     W2R_CUDA(cudaMemsetAsync(d->quals + d->quals_bytes, 0, 32, s));
     const double t2 = now_ms();
     if (n) {
-        const unsigned nbatch = (batched && n >= (1u << 20)) ? 8u : 1u;
+        const unsigned nbatch = forced_batches ? (unsigned)forced_batches : (batched && n >= (1u << 20)) ? 8u : 1u;
         for (unsigned b = 0; b < nbatch; ++b) {
             const uint64_t r0 = n * b / nbatch, r1 = n * (b + 1) / nbatch;
             const uint64_t b0 = in->base_off[r0], b1 = in->base_off[r1], q0 = in->qual_off[r0], q1 = in->qual_off[r1];
