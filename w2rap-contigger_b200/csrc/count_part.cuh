@@ -11,7 +11,9 @@
 //                                 shared-memory hash table.  The partition's records are staged into shared memory by bulk
 //                                 asynchronous copies (cp.async.bulk + mbarrier, double buffered; SASS: UBLKCP/SYNCS), and the
 //                                 warps expand them FLAT: lane l takes k-mer t + l of a group of 32 records, so every lane forms and
-//                                 inserts a k-mer whatever the record lengths.  Then histogram + solid records.
+//                                 inserts a k-mer whatever the record lengths.  Then histogram + solid records, sorted by
+//                                 (minimiser, offset of the minimiser) so that the k-mers of a chain leave next to each other:
+//                                 their index in the solid array is their node id in the graph stage (unipath.cuh: DenseNodes).
 //           k_count_region /    : fallback for partitions whose distinct k-mers do not fit shared memory: inserts into a 32 MB
 //           k_scan_region         table region that stays resident in L2 (128-bit CAS, count/context REDs), then scan + reset.
 // DRAM traffic: 32 B written + 32 B read per RECORD (~13-18 k-mers) and nothing else; the same records cross NVLink when sharded.
@@ -315,6 +317,8 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
     __shared__ unsigned int sh_hist[104];
     __shared__ int sh_fail;
     __shared__ uint32_t sh_tot[2], sh_cnt[2];                   // per staging buffer: records of the whole partition / of the staged chunk
+    __shared__ uint32_t sh_nsolid;                              // solid k-mers of the partition
+    __shared__ unsigned long long sh_solid_base;                // where they go in solid_out
     const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
     const unsigned le_mask = (2u << lane) - 1u;                 // lanes 0..lane
     for (int j = threadIdx.x; j < 104; j += blockDim.x) sh_hist[j] = 0;
@@ -368,7 +372,7 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
             uint4* cw = reinterpret_cast<uint4*>(ccs);
             for (uint32_t j = threadIdx.x; j < SMEM_SLOTS / 4; j += blockDim.x) cw[j] = make_uint4(0, 0, 0, 0);
         }
-        if (threadIdx.x == 0) sh_fail = 0;
+        if (threadIdx.x == 0) { sh_fail = 0; sh_nsolid = 0; }
         __syncthreads();
         auto insert = [&](const Kmer k, const uint32_t ctx) {
             uint32_t s = smem_slot_hash(k) >> (32 - sp.log_slots);
@@ -445,6 +449,7 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
         if (failed) {
             if (threadIdx.x == 0) sp.failed[atomicAdd(sp.failed_cursor, 1ull)] = p;
         } else {
+            // 1. histogram and dump; a solid key takes its context into the free low byte of w1, every other key is cleared
             for (uint32_t base = 0; base < SMEM_SLOTS; base += blockDim.x) {
                 const uint32_t j = base + threadIdx.x;
                 const bool in = j < SMEM_SLOTS;
@@ -457,13 +462,78 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
                 const unsigned ones = __ballot_sync(0xffffffffu, occ && c == 1u);
                 if (lane == 0 && ones) atomicAdd(&sh_hist[1], (unsigned)__popc(ones));
                 if (occ && c != 1u) atomicAdd(&sh_hist[c > 100u ? 100u : c], 1u);
-                const bool solid = occ && c >= sp.min_freq;
-                const uint64_t pos = warp_append(sp.solid_cursor, solid);
-                if (solid) { if (pos < sp.solid_cap) sp.solid_out[pos] = make_ulonglong2(kk.x, kk.y | ctx); else atomicExch(sp.solid_overflow, 1); }
+                if (occ) keys[j] = c >= sp.min_freq ? make_ulonglong2(kk.x, kk.y | ctx) : make_ulonglong2(~0ull, ~0ull);
                 if (sp.dump_out) {
                     const uint64_t dp = warp_append(sp.dump_cursor, occ);
                     if (occ) sp.dump_out[dp] = DumpRec{kk.x, kk.y, c, ctx, NIL, 0};
                 }
+            }
+            __syncthreads();
+            // 2. the solid slots, compacted into the (now free) count array
+            for (uint32_t base = 0; base < SMEM_SLOTS; base += blockDim.x) {
+                const uint32_t j = base + threadIdx.x;
+                const bool solid = j < SMEM_SLOTS && keys[j].x != ~0ull;
+                const unsigned m = __ballot_sync(0xffffffffu, solid);
+                uint32_t first = 0;
+                if (lane == 0 && m) first = atomicAdd(&sh_nsolid, (uint32_t)__popc(m));
+                first = __shfl_sync(0xffffffffu, first, 0);
+                if (solid) ccs[first + __popc(m & (le_mask >> 1))] = j;
+            }
+            __syncthreads();
+            // 3. one sort word per solid k-mer, in place (after the compaction every lane that computes a minimiser has a k-mer):
+            // minimiser bits : 13 | offset : 6 | slot : 13
+            const uint32_t ns = sh_nsolid, N = ns <= 1u ? ns : 1u << (32 - __clz(ns - 1u));
+            for (uint32_t i = threadIdx.x; i < ns; i += blockDim.x) {
+                const uint32_t j = ccs[i];
+                const ulonglong2 kk = keys[j];
+                uint32_t off;
+                const uint32_t mh = kmer_minimizer_offset_words(Kmer{kk.x, kk.y & ~0xffull}, &off);
+                ccs[i] = (mh & 0x1fffu) << 19 | off << 13 | j;
+            }
+            // 4. bitonic sort, ascending, over the next power of two (the pad words sort last)
+            if (N <= blockDim.x) {
+                // one word per thread in a register: pairs less than 32 apart meet by shuffles, wider ones through shared memory
+                const uint32_t i = threadIdx.x;
+                __syncthreads();
+                uint32_t v = i < ns ? ccs[i] : ~0u;
+                for (uint32_t kb = 2; kb <= N; kb <<= 1) {
+                    for (uint32_t jb = kb >> 1; jb > 0; jb >>= 1) {
+                        uint32_t o;
+                        if (jb >= 32u) {
+                            __syncthreads();
+                            if (i < N) ccs[i] = v;
+                            __syncthreads();
+                            o = i < N ? ccs[i ^ jb] : ~0u;
+                        } else o = __shfl_xor_sync(0xffffffffu, v, jb);
+                        const bool keep_min = ((i & jb) == 0) == ((i & kb) == 0);
+                        v = keep_min ? (v < o ? v : o) : (v < o ? o : v);
+                    }
+                }
+                __syncthreads();
+                if (i < N) ccs[i] = v;
+            } else {
+                // in shared memory: a substage whose pairs are at most 32 apart stays inside one warp's 64 words, so only the wider
+                // ones need the whole CTA at a barrier
+                for (uint32_t i = ns + threadIdx.x; i < N; i += blockDim.x) ccs[i] = ~0u;
+                __syncthreads();
+                for (uint32_t kb = 2; kb <= N; kb <<= 1) {
+                    for (uint32_t jb = kb >> 1; jb > 0; jb >>= 1) {
+                        if (jb > 32u) __syncthreads();
+                        for (uint32_t t = threadIdx.x; t < N / 2; t += blockDim.x) {
+                            const uint32_t i = 2 * t - (t & (jb - 1u));
+                            const uint32_t a = ccs[i], b = ccs[i + jb];
+                            if ((a > b) == ((i & kb) == 0)) { ccs[i] = b; ccs[i + jb] = a; }
+                        }
+                        if (jb > 32u) __syncthreads(); else __syncwarp();
+                    }
+                }
+            }
+            // 5. one cursor atomic per partition, the records in sorted order
+            if (threadIdx.x == 0 && ns) sh_solid_base = atomicAdd(sp.solid_cursor, (unsigned long long)ns);
+            __syncthreads();
+            for (uint32_t i = threadIdx.x; i < ns; i += blockDim.x) {
+                const uint64_t pos = sh_solid_base + i;
+                if (pos < sp.solid_cap) sp.solid_out[pos] = keys[ccs[i] & 0x1fffu]; else atomicExch(sp.solid_overflow, 1);
             }
         }
         __syncthreads();

@@ -103,11 +103,11 @@ W2R_HD void skm_kmer_at(const uint64_t* q, uint32_t j, Kmer* canon, uint32_t* ct
 constexpr int MINI_M = 15;
 constexpr int MINI_W = K - MINI_M + 1;     // m-mers per k-mer
 // hash of the canonical m-mer starting at base `pos` (a bijection of its 30-bit value, so equal hash <=> equal canonical m-mer)
+W2R_HD uint32_t mmer_rc(uint32_t v) { return rev2_32(~v) >> (32 - 2 * MINI_M); }             // reverse complement, same encoding
+W2R_HD uint32_t mmer_mix(uint32_t c) { c ^= c >> 16; c *= 0x85ebca6bu; c ^= c >> 13; c *= 0xc2b2ae35u; c ^= c >> 16; return c; }
 W2R_HD uint32_t mmer_hash_of(uint32_t v) {                                                   // v: the m-mer, first base in bits 1:0
-    const uint32_t rc = rev2_32(~v) >> (32 - 2 * MINI_M);                                    // reverse complement, same encoding
-    uint32_t c = v < rc ? v : rc;
-    c ^= c >> 16; c *= 0x85ebca6bu; c ^= c >> 13; c *= 0xc2b2ae35u; c ^= c >> 16;
-    return c;
+    const uint32_t rc = mmer_rc(v);
+    return mmer_mix(v < rc ? v : rc);
 }
 W2R_HD uint32_t mmer_hash_at(const uint8_t* bases, uint64_t pos) { return mmer_hash_of(bases16_at(bases, pos) & ((1u << (2 * MINI_M)) - 1u)); }
 // window minima are biased towards 0: re-mix before taking partition bits (top) and pass bits (low 16)
@@ -128,6 +128,30 @@ W2R_HD uint32_t kmer_minimizer_hash_words(Kmer k) {
         const uint32_t h = mmer_hash_of((uint32_t)w & ((1u << (2 * MINI_M)) - 1u));
         if (h < m) m = h;
     }
+    return m;
+}
+// The same minimiser hash, and in *offset where the minimiser sits, normalised for strand: q if the canonical m-mer occurs forward
+// at base q of k, MINI_W - 1 - q if it occurs reverse-complemented there.  A k-mer and its reverse complement get the same offset,
+// and along a stretch of genome that keeps its minimiser the offset steps by exactly one per k-mer, whichever strand each k-mer is
+// stored in: sorting a partition's k-mers by (minimiser, offset) puts the k-mers of a chain next to each other (the reduce does
+// that, count_part.cuh).  A minimiser that occurs twice takes the smaller offset, which keeps the offset strand-symmetric.
+W2R_HD uint32_t mmer_bits_at(uint64_t lo, uint64_t hi, int bit) {        // the 15 bases from 2-bit group bit/2 of hi:lo
+    const uint64_t w = bit == 0 ? lo : (bit < 64 ? (lo >> bit) | (hi << (64 - bit)) : hi >> (bit - 64));
+    return (uint32_t)w & ((1u << (2 * MINI_M)) - 1u);
+}
+W2R_HD uint32_t kmer_minimizer_offset_words(Kmer k, uint32_t* offset) {
+    const uint64_t lo = rev2(k.w0), hi = rev2(k.w1);                  // the k-mer LSB-first (base i in bits 2i..2i+1 of hi:lo)
+    const uint64_t rlo = (~k.w1 >> 8) | (~k.w0 << 56), rhi = ~k.w0 >> 8; // its reverse complement LSB-first: the complement moved down 8
+    uint32_t m = 0xffffffffu, off = 0;
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (int t = 0; t < MINI_W; ++t) {
+        const uint32_t v = mmer_bits_at(lo, hi, 2 * t), rc = mmer_bits_at(rlo, rhi, 2 * (MINI_W - 1 - t));   // rc == mmer_rc(v)
+        const uint32_t h = mmer_mix(v < rc ? v : rc), o = v < rc ? (uint32_t)t : (uint32_t)(MINI_W - 1 - t);
+        if (h < m || (h == m && o < off)) { m = h; off = o; }
+    }
+    *offset = off;
     return m;
 }
 // reference form for tests: the minimiser hash of the k-mer starting at base j

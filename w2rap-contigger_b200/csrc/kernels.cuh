@@ -3,8 +3,8 @@
 // K1 k_good_len                    : PQVec quality floor (count_part.cuh: k_minimizer_map = k-mer extraction + partition by minimiser)
 // K2 k_count_smem, k_count_region / k_scan_region (count_part.cuh) : count per partition in shared memory / in an L2-resident
 //    region, histogram, min-frequency filter; k_insert_solid
-// K3 k_adjacency                  : recomputeAdjacencies
-// K4 k_links / k_rank_* / k_cycle_* / k_strand_decide / k_collect_heads / k_assign_edges / k_emit_edges : unipaths
+// K3 k_adjacency_dense / k_adjacency : recomputeAdjacencies (over the dense nodes of one GPU / the local table of a sharded run)
+// K4 k_links / k_rank_* / k_cycle_* / k_strand_decide / k_collect_heads / k_assign_edges / k_emit_edges / k_backfill_slots : unipaths
 // K5 k_edge_ends / k_vertex_* / k_hbv_edges / k_adj_* : HBV vertices + incidence
 // K6 k_path_reads / k_path_gather : read pathing (+FixPaths)
 #pragma once
@@ -108,7 +108,9 @@ __global__ void k_dump_solid(SolidTable st, DumpRec* __restrict__ out, unsigned 
 
 // Dictionary build (BuildReadQGraph.cc:1096-1104 insertEntryNoLocking, in parallel): keys are unique, so a successful CAS owns the slot.
 // bloom (optional): the pathing filter's bits are set on the way (kmer.cuh: PathDict), which saves a sweep over the finished table.
-__global__ void k_insert_solid(const ulonglong2* __restrict__ recs, uint64_t n, SolidTable st, uint32_t* __restrict__ bloom, uint32_t bloom_W, uint32_t slice_words) {
+// dense (optional, one GPU): record i also becomes node i of the graph stage (unipath.cuh: DenseNodes), and its slot's `off` holds i.
+__global__ void k_insert_solid(const ulonglong2* __restrict__ recs, uint64_t n, SolidTable st, uint32_t* __restrict__ bloom, uint32_t bloom_W, uint32_t slice_words,
+                               SolidSlot* __restrict__ dense) {
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
         ulonglong2 rec = __ldcs(recs + i);
         Kmer k{rec.x, rec.y & ~0xffull};
@@ -118,9 +120,10 @@ __global__ void k_insert_solid(const ulonglong2* __restrict__ recs, uint64_t n, 
         for (;;) {
             SolidSlot* p = st.slots + h;
             U128 old = cas128(p, ~0ull, ~0ull, k.w0, k.w1);
-            if (old.lo == ~0ull && old.hi == ~0ull) { p->ctx = ctx; p->edge = NIL; p->off = 0; p->pad = 0; break; }
+            if (old.lo == ~0ull && old.hi == ~0ull) { p->ctx = ctx; p->edge = NIL; p->off = dense ? (uint32_t)i : 0u; p->pad = 0; break; }
             h = st.next(h);
         }
+        if (dense) dense[i] = SolidSlot{k.w0, k.w1, ctx, NIL, 0, 0};
     }
 }
 // The same from whole entries (k-mer, pruned context, edge, offset): the pathing dictionary of a sharded run is built from the
@@ -150,9 +153,18 @@ __global__ void k_adjacency(SolidTable st) {
         if (c2 != c) s->ctx = c2;     // other threads only test membership (keys), never contexts, during this kernel
     }
 }
+// The same over the dense nodes (one GPU): a sequential sweep; the neighbours are probed in the table.
+__global__ void k_adjacency_dense(DenseNodes d) {
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < d.n; i += (uint64_t)gridDim.x * blockDim.x) {
+        SolidSlot* s = d.nodes + i;
+        const uint32_t c = s->ctx & 0xffu, c2 = pruned_context(d.t, Kmer{s->w0, s->w1}, c);
+        if (c2 != c) s->ctx = c2;
+    }
+}
 
 // ================================================================ K4: unipaths
-__global__ void k_links(SolidTable st, uint32_t* __restrict__ next0, int* __restrict__ missing) {
+template <class V>
+__global__ void k_links(V st, uint32_t* __restrict__ next0, int* __restrict__ missing) {
     const uint64_t nn = 2 * st.size();
     for (uint64_t x = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; x < nn; x += (uint64_t)gridDim.x * blockDim.x) {
         int miss = 0;
@@ -253,7 +265,8 @@ __global__ void k_cycle_init(const uint32_t* __restrict__ list, uint64_t n, cons
         A[x] = RankState{next0[x], x >> 1};
     }
 }
-__global__ void k_cycle_step(const uint32_t* __restrict__ list, uint64_t n, SolidTable st, const RankState* __restrict__ A, RankState* __restrict__ B, int* __restrict__ changed) {
+template <class V>
+__global__ void k_cycle_step(const uint32_t* __restrict__ list, uint64_t n, V st, const RankState* __restrict__ A, RankState* __restrict__ B, int* __restrict__ changed) {
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
         uint32_t x = list[i];
         bool ch;
@@ -269,13 +282,15 @@ __global__ void k_cycle_cut(const uint32_t* __restrict__ list, uint64_t n, const
 }
 // Per strand path: keep it iff its sequence is FWD or PALINDROME (dna/CanonicalForm.h:34-46, BuildReadQGraph.cc:247-258).
 // R[x] = (tail(x), dist to tail | RESOLVED).  keep[] is indexed by the head node of the strand.
-__global__ void k_strand_decide(SolidTable st, const RankState* __restrict__ R, uint8_t* __restrict__ keep, int* __restrict__ too_long) {
+template <class V>
+__global__ void k_strand_decide(V st, const RankState* __restrict__ R, uint8_t* __restrict__ keep, int* __restrict__ too_long) {
     const uint64_t nn = 2 * st.size();
     for (uint64_t xi = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; xi < nn; xi += (uint64_t)gridDim.x * blockDim.x) {
         if (strand_decide_node(st, R, (uint32_t)xi, keep)) atomicExch(too_long, 1);
     }
 }
-__global__ void k_collect_heads(SolidTable st, const RankState* __restrict__ R, const uint8_t* __restrict__ keep, uint32_t* __restrict__ h_node,
+template <class V>
+__global__ void k_collect_heads(V st, const RankState* __restrict__ R, const uint8_t* __restrict__ keep, uint32_t* __restrict__ h_node,
                                 uint64_t* __restrict__ h_w0, uint64_t* __restrict__ h_w1, uint32_t* __restrict__ h_n, unsigned long long* cursor, uint64_t cap) {
     const uint64_t nn = 2 * st.size();
     for (uint64_t base = (uint64_t)blockIdx.x * blockDim.x; base < nn; base += (uint64_t)gridDim.x * blockDim.x) {
@@ -308,11 +323,23 @@ struct OrBase {
     }
 };
 // Every k-mer of a kept strand writes its first base (the tail also its other 59) and its KDef (edge id, offset).
-__global__ void k_emit_edges(SolidTable st, const RankState* __restrict__ R, const uint32_t* __restrict__ edge_of_head, const uint64_t* __restrict__ edge_off,
+template <class V>
+__global__ void k_emit_edges(V st, const RankState* __restrict__ R, const uint32_t* __restrict__ edge_of_head, const uint64_t* __restrict__ edge_off,
                              uint8_t* __restrict__ edge_bases) {
     const uint64_t nn = 2 * st.size();
     OrBase put{edge_bases};
     for (uint64_t xi = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; xi < nn; xi += (uint64_t)gridDim.x * blockDim.x) emit_node(st, R, edge_of_head, edge_off, (uint32_t)xi, put);
+}
+// After the graph stage over dense nodes: every table slot takes its node's pruned context, edge and offset, so the pathing
+// dictionary and the dump see the table they always saw.
+__global__ void k_backfill_slots(SolidTable st, const SolidSlot* __restrict__ dense) {
+    const uint64_t T = st.size();
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < T; i += (uint64_t)gridDim.x * blockDim.x) {
+        SolidSlot* s = st.slots + i;
+        if (s->w0 == EMPTY_W0) continue;
+        const SolidSlot& d = dense[s->off];
+        s->ctx = d.ctx; s->edge = d.edge; s->off = d.off;
+    }
 }
 
 // Device -> pinned host memory by stores over PCIe instead of the copy engine: the D2H engine is shared by every stream, and the

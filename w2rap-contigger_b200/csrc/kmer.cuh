@@ -170,7 +170,7 @@ struct __attribute__((aligned(32))) SolidSlot { uint64_t w0, w1; uint32_t ctx, e
 struct SolidTable {
     SolidSlot* slots;
     uint64_t nslots;           // any size (not only powers of two): the home slot is the hash scaled to [0, nslots).  Tables whose slots
-                               // become 32-bit oriented node ids (2*slot+o: the graph stage) hold <= 2^31 slots; the pathing table any number
+                               // become 32-bit oriented node ids (2*slot+o: the sharded graph stage) hold <= 2^31 slots; the pathing table any number
     W2R_HD uint64_t size() const { return nslots; }
     W2R_HD uint64_t home_of_hash(uint64_t h) const { return mulhi64(h, nslots); }
     W2R_HD uint64_t home(Kmer k) const { return home_of_hash(kmer_hash(k)); }

@@ -1,7 +1,7 @@
 // unipath.cuh — unipath (edge) structure over the solid k-mer table, restated for data-parallel execution.
 //
 // The reference walks edges serially from their ends (EdgeBuilder, paths/long/BuildReadQGraph.cc:99-339).  Here every
-// solid k-mer is two ORIENTED nodes, node id = 2*slot + o (o = 1: the node spells rc(key[slot])).  A successor link
+// solid k-mer is two ORIENTED nodes, node id = 2*id + o (o = 1: the node spells rc(key[id]); DenseNodes below says what an id is).  A successor link
 // x -> n exists iff the reference's walk would step from x to n:
 //     x is not a palindrome, x has exactly one successor n, n is not a palindrome, n has exactly one predecessor
 //     (extend(): :234-246; the same test seen from n is upstreamExtensionPossible(): :192-202).
@@ -21,8 +21,29 @@ constexpr uint32_t GHOST_TAIL = 0xfffffffdu;   // next0[] of a GHOST node (shard
                                                // rank owns.  A node whose successor is a ghost is the tail of its LOCAL chain piece.
 W2R_HD bool slot_is_ghost(const SolidSlot& s) { return s.pad != 0; }      // pad = owner rank + 1, edge = slot on the owner
 
-W2R_HD Kmer node_kmer(const SolidTable& t, uint32_t x) {
-    const SolidSlot& s = t.slots[x >> 1];
+// How nodes are numbered: oriented node = 2*id + o, and a node view maps an id to its entry (k-mer, context, edge, offset) and a
+// canonical k-mer to its id.  Both views probe the same hash table for neighbours.
+//   SolidTable : id = slot of the table.  The sharded graph stage numbers its nodes so (its ghosts live in the local table).
+//   DenseNodes : id = index in the dense array of solid k-mers, in the order the reduce emitted them: grouped by minimiser and
+//                sorted by the minimiser's place (count_part.cuh), so the k-mers of a chain mostly get neighbouring ids and a chain
+//                step stays inside a sector or two.  The table's `off` field holds every key's id until the graph stage ends.
+struct DenseNodes {
+    SolidTable t;
+    SolidSlot* nodes;
+    uint64_t n;
+    W2R_HD uint64_t size() const { return n; }
+};
+W2R_HD SolidSlot& node_entry(const SolidTable& t, uint64_t id) { return t.slots[id]; }
+W2R_HD SolidSlot& node_entry(const DenseNodes& d, uint64_t id) { return d.nodes[id]; }
+W2R_HD int64_t node_find(const SolidTable& t, Kmer k) { return solid_find(t, k); }
+W2R_HD int64_t node_find(const DenseNodes& d, Kmer k) {
+    const int64_t s = solid_find(d.t, k);
+    return s < 0 ? -1 : (int64_t)d.t.slots[s].off;
+}
+
+template <class V>
+W2R_HD Kmer node_kmer(const V& v, uint32_t x) {
+    const SolidSlot& s = node_entry(v, x >> 1);
     Kmer k{s.w0, s.w1};
     return (x & 1u) ? kmer_rc(k) : k;
 }
@@ -30,8 +51,9 @@ W2R_HD Kmer node_kmer(const SolidTable& t, uint32_t x) {
 // Successor link of oriented node x, or NIL.  *missing is set if a neighbour that the pruned context promises is absent
 // (the reference would ForceAssert, :265).
 // *to_ghost (optional) is set if the successor is a ghost node.
-W2R_HD uint32_t unipath_succ_link(const SolidTable& t, uint32_t x, int* missing, bool* to_ghost = nullptr) {
-    const SolidSlot& s = t.slots[x >> 1];
+template <class V>
+W2R_HD uint32_t unipath_succ_link(const V& t, uint32_t x, int* missing, bool* to_ghost = nullptr) {
+    const SolidSlot& s = node_entry(t, x >> 1);
     if (to_ghost) *to_ghost = false;
     if (s.w0 == EMPTY_W0) return EMPTY_NODE;
     if (slot_is_ghost(s)) return GHOST_TAIL;
@@ -46,12 +68,12 @@ W2R_HD uint32_t unipath_succ_link(const SolidTable& t, uint32_t x, int* missing,
     Kmer nrc = kmer_rc(n);
     if (nrc == n) return NIL;                                   // :239
     bool rev = kmer_less(nrc, n);
-    int64_t ts = solid_find(t, rev ? nrc : n);
+    int64_t ts = node_find(t, rev ? nrc : n);
     if (ts < 0) { if (missing) *missing = 1; return NIL; }
-    uint32_t c2 = t.slots[ts].ctx & 0xffu;
+    uint32_t c2 = node_entry(t, ts).ctx & 0xffu;
     if (rev) c2 = ctx_rc(c2);
     if (nib_count(c2 >> 4) != 1) return NIL;                    // :242
-    if (to_ghost) *to_ghost = slot_is_ghost(t.slots[ts]);
+    if (to_ghost) *to_ghost = slot_is_ghost(node_entry(t, ts));
     return (uint32_t)(2 * ts) + (rev ? 1u : 0u);
 }
 
@@ -121,12 +143,13 @@ W2R_HD RankState rank_step_node(const RankState* A, uint32_t x, bool* unresolved
     }
     return a;
 }
-// Smooth circles: state = (jump pointer, slot of the minimum canonical k-mer seen so far).
-W2R_HD RankState cycle_step_node(const SolidTable& t, const RankState* A, uint32_t x, bool* changed) {
+// Smooth circles: state = (jump pointer, id of the minimum canonical k-mer seen so far).
+template <class V>
+W2R_HD RankState cycle_step_node(const V& t, const RankState* A, uint32_t x, bool* changed) {
     RankState a = A[x], b = A[a.x];
     uint32_t best = a.y;
     if (b.y != a.y) {
-        const SolidSlot& sa = t.slots[a.y]; const SolidSlot& sb = t.slots[b.y];
+        const SolidSlot& sa = node_entry(t, a.y); const SolidSlot& sb = node_entry(t, b.y);
         if (kmer_less(Kmer{sb.w0, sb.w1}, Kmer{sa.w0, sa.w1})) best = b.y;
     }
     *changed = best != a.y;
@@ -142,8 +165,9 @@ W2R_HD void cycle_cut_node(const RankState* A, uint32_t* next0, uint32_t x) {
 }
 // Strand selection (dna/CanonicalForm.h:34-46, BuildReadQGraph.cc:247-258): R[x] = (tail, distance to tail); keep[] is indexed
 // by the head node of a strand path.  Returns true if the strand is longer than KDef's 24-bit offset allows.
-W2R_HD bool strand_decide_node(const SolidTable& t, const RankState* R, uint32_t x, uint8_t* keep) {
-    if (t.slots[x >> 1].w0 == EMPTY_W0) return false;
+template <class V>
+W2R_HD bool strand_decide_node(const V& t, const RankState* R, uint32_t x, uint8_t* keep) {
+    if (node_entry(t, x >> 1).w0 == EMPTY_W0) return false;
     RankState a = R[x], f = R[x ^ 1u];
     uint32_t d = a.y & ~RANK_RESOLVED, off = f.y & ~RANK_RESOLVED;
     uint64_t n = (uint64_t)d + off + 1;
@@ -159,13 +183,14 @@ W2R_HD bool strand_decide_node(const SolidTable& t, const RankState* R, uint32_t
     }
     return off == 0 && n > 0x1000000ull;                 // offsets must fit KDef's 24 bits (kmers/ReadPather.h:121-122,144)
 }
-W2R_HD bool head_is_kept(const SolidTable& t, const RankState* R, const uint8_t* keep, uint32_t x) {
-    return t.slots[x >> 1].w0 != EMPTY_W0 && (R[x ^ 1u].y & ~RANK_RESOLVED) == 0 && keep[x];
+template <class V>
+W2R_HD bool head_is_kept(const V& t, const RankState* R, const uint8_t* keep, uint32_t x) {
+    return node_entry(t, x >> 1).w0 != EMPTY_W0 && (R[x ^ 1u].y & ~RANK_RESOLVED) == 0 && keep[x];
 }
 // Edge emission + KDef back-fill for one node (BuildReadQGraph.cc:287-301).  put(edge byte offset, base position, base code).
-template <class Put>
-W2R_HD void emit_node(const SolidTable& t, const RankState* R, const uint32_t* edge_of_head, const uint64_t* edge_off, uint32_t x, Put& put) {
-    SolidSlot* s = t.slots + (x >> 1);
+template <class V, class Put>
+W2R_HD void emit_node(const V& t, const RankState* R, const uint32_t* edge_of_head, const uint64_t* edge_off, uint32_t x, Put& put) {
+    SolidSlot* s = &node_entry(t, x >> 1);
     if (s->w0 == EMPTY_W0) return;
     RankState f = R[x ^ 1u];
     uint32_t e = edge_of_head[f.x ^ 1u];
