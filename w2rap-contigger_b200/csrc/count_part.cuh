@@ -19,6 +19,7 @@
 // DRAM traffic: 32 B written + 32 B read per RECORD (~13-18 k-mers) and nothing else; the same records cross NVLink when sharded.
 #pragma once
 #include "kernels.cuh"
+#include "prims.cuh"
 #include "shard.cuh"
 
 namespace w2r {
@@ -255,6 +256,7 @@ struct SmemCountParams {
     uint32_t log_slots;                                        // table size of this launch
     uint32_t chunk;                                            // records per staging buffer (two buffers); <= SKM_CHUNK
     const uint32_t* plist; uint32_t nlist;                     // if set: only these partitions (the ones a smaller table could not hold)
+    uint8_t* count_out;                                        // k_count_smem<true>: min(255, count) of solid_out[i] at count_out[i]
 };
 
 // --- mbarrier + bulk-copy wrappers (PTX; SASS: SYNCS.*, UBLKCP)
@@ -306,6 +308,8 @@ __device__ __forceinline__ ulonglong2 lds128_volatile(const void* addr) {
     return v;
 }
 
+// KEEP_COUNTS (w2rap_step2_count): also write min(255, count) of every emitted record to sp.count_out, parallel to solid_out.
+template <bool KEEP_COUNTS>
 __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const uint32_t SMEM_SLOTS = 1u << sp.log_slots;
@@ -445,6 +449,13 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
             __syncthreads();                                     // chunk consumed (and, after the last one, every insert has landed)
             if (!more) { ++it; break; }
         }
+        // KEEP_COUNTS: the count of slot j is stashed at kept[j] from step 1 to step 5, because the sort word of step 3
+        // (minimiser 13 | offset 6 | slot 13) has no room for it and the key's spare byte holds the context.  kept[] is the staging
+        // buffer this partition's last chunk came through (buffer (it - 1) & 1): the barrier above was the last read of it, the
+        // bulk copy into it has completed (waited on), and the next partition's chunk 0 is already in flight into the OTHER buffer.
+        // Nothing is issued into this one before the next partition's first chunk has been waited for, which is after the barrier
+        // that ends this partition.  It holds CHUNK * 32 >= 16 KB; the counts take SMEM_SLOTS <= 8 KB.
+        uint8_t* kept = reinterpret_cast<uint8_t*>(stage + (size_t)((it - 1u) & 1u) * CHUNK);
         const bool failed = sh_fail != 0;
         if (failed) {
             if (threadIdx.x == 0) sp.failed[atomicAdd(sp.failed_cursor, 1ull)] = p;
@@ -463,6 +474,7 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
                 if (lane == 0 && ones) atomicAdd(&sh_hist[1], (unsigned)__popc(ones));
                 if (occ && c != 1u) atomicAdd(&sh_hist[c > 100u ? 100u : c], 1u);
                 if (occ) keys[j] = c >= sp.min_freq ? make_ulonglong2(kk.x, kk.y | ctx) : make_ulonglong2(~0ull, ~0ull);
+                if (KEEP_COUNTS && in) kept[j] = (uint8_t)c;
                 if (sp.dump_out) {
                     const uint64_t dp = warp_append(sp.dump_cursor, occ);
                     if (occ) sp.dump_out[dp] = DumpRec{kk.x, kk.y, c, ctx, NIL, 0};
@@ -533,7 +545,11 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
             __syncthreads();
             for (uint32_t i = threadIdx.x; i < ns; i += blockDim.x) {
                 const uint64_t pos = sh_solid_base + i;
-                if (pos < sp.solid_cap) sp.solid_out[pos] = keys[ccs[i] & 0x1fffu]; else atomicExch(sp.solid_overflow, 1);
+                if (pos < sp.solid_cap) {
+                    const uint32_t j = ccs[i] & 0x1fffu;
+                    sp.solid_out[pos] = keys[j];
+                    if (KEEP_COUNTS) sp.count_out[pos] = kept[j];
+                } else atomicExch(sp.solid_overflow, 1);
             }
         }
         __syncthreads();
@@ -554,6 +570,7 @@ struct ScanParams {
     unsigned long long* dump_cursor;
     const int* overflow;             // if set: the group failed, only reset the region
     int* solid_overflow;
+    uint8_t* count_out;              // or nullptr; else min(255, count) of solid_out[i] goes to count_out[i] (w2rap_step2_count)
 };
 // hist[min(100,min(255,count))]++ (BuildReadQGraph.cc:1094-1097), keep count >= minFreq (:1098), reset the region.
 __global__ void __launch_bounds__(256) k_scan_region(ScanParams sp) {
@@ -583,7 +600,10 @@ __global__ void __launch_bounds__(256) k_scan_region(ScanParams sp) {
         if (occ && (peers & ((1u << lane_id()) - 1u)) == 0) atomicAdd(&sh[bin], (unsigned)__popc(peers));
         solid = occ && c >= sp.min_freq;
         uint64_t pos = warp_append(sp.solid_cursor, solid);
-        if (solid) { if (pos < sp.solid_cap) sp.solid_out[pos] = make_ulonglong2(k.x, k.y | ctx); else atomicExch(sp.solid_overflow, 1); }
+        if (solid) {
+            if (pos < sp.solid_cap) { sp.solid_out[pos] = make_ulonglong2(k.x, k.y | ctx); if (sp.count_out) sp.count_out[pos] = (uint8_t)c; }
+            else atomicExch(sp.solid_overflow, 1);
+        }
         if (sp.dump_out) {
             uint64_t dp = warp_append(sp.dump_cursor, occ);
             if (occ) sp.dump_out[dp] = DumpRec{k.x, k.y, c, ctx, NIL, 0};
@@ -593,6 +613,40 @@ __global__ void __launch_bounds__(256) k_scan_region(ScanParams sp) {
     if (!failed) {
         for (int j = threadIdx.x; j <= 100; j += blockDim.x) if (sh[j]) atomicAdd(&sp.hist[j], (unsigned long long)sh[j]);
     }
+}
+
+// ---------------------------------------------------------------- selection from kept counts (w2rap_step2_build)
+// The records a count kept (every k-mer seen >= f0 times, in the reduce's order) with count >= min_freq, compacted STABLY into
+// the solid array: the reduce emits each partition's records sorted by minimiser and offset, and that order gives the k-mers of a
+// chain neighbouring node ids in the graph stage (unipath.cuh: DenseNodes).  An append by warp aggregation would scramble it.
+// Tile t = records [t * SCAN_TILE, +SCAN_TILE), thread i of it holds the SCAN_ITEMS consecutive records from i * SCAN_ITEMS (one
+// 8-byte load of their counts): selected per tile, an exclusive scan of the tile sums (prims.cuh), then an in-order scatter.
+static_assert(SCAN_ITEMS == 8, "one 8-byte load of counts per thread");
+__device__ __forceinline__ uint32_t select_mask(const uint8_t* __restrict__ count, uint64_t n, uint64_t base, uint32_t min_freq) {
+    uint32_t m = 0;
+    if (base + SCAN_ITEMS <= n) {
+        const uint64_t w = *reinterpret_cast<const uint64_t*>(count + base);
+#pragma unroll
+        for (int i = 0; i < SCAN_ITEMS; ++i) if (((w >> (8 * i)) & 0xffu) >= min_freq) m |= 1u << i;
+    } else {
+        for (int i = 0; base + i < n; ++i) if (count[base + i] >= min_freq) m |= 1u << i;
+    }
+    return m;
+}
+__global__ void __launch_bounds__(SCAN_THREADS) k_select_tile_counts(const uint8_t* __restrict__ count, uint64_t n, uint32_t min_freq, uint32_t* __restrict__ tile_n) {
+    __shared__ uint32_t sm[33];
+    const uint64_t base = (uint64_t)blockIdx.x * SCAN_TILE + (uint64_t)threadIdx.x * SCAN_ITEMS;
+    uint32_t total;
+    block_exclusive_scan<uint32_t>((uint32_t)__popc(select_mask(count, n, base, min_freq)), &total, sm);
+    if (threadIdx.x == 0) tile_n[blockIdx.x] = total;
+}
+__global__ void __launch_bounds__(SCAN_THREADS) k_select_solid(const ulonglong2* __restrict__ kept, const uint8_t* __restrict__ count, uint64_t n, uint32_t min_freq,
+                                                               const uint64_t* __restrict__ tile_base, ulonglong2* __restrict__ solid) {
+    __shared__ uint32_t sm[33];
+    const uint64_t base = (uint64_t)blockIdx.x * SCAN_TILE + (uint64_t)threadIdx.x * SCAN_ITEMS;
+    uint32_t m = select_mask(count, n, base, min_freq), total;
+    uint64_t pos = tile_base[blockIdx.x] + block_exclusive_scan<uint32_t>((uint32_t)__popc(m), &total, sm);
+    for (; m; m &= m - 1u) solid[pos++] = kept[base + (uint32_t)(__ffs((int)m) - 1)];
 }
 
 }  // namespace w2r

@@ -3,6 +3,8 @@
 // Mirrors buildReadQGraph (paths/long/BuildReadQGraph.cc:1253-1327) stage by stage:
 //   createDictOMPRecursive  -> count_stage()      (k_good_len, k_minimizer_map x2, [NCCL exchange], k_count_smem, k_count_region + k_scan_region as
 //                                                  fallback, k_insert_solid)
+//                           -> select_stage()     (w2rap_step2_build: k_select_tile_counts, scan, k_select_solid over the counts that
+//                                                  w2rap_step2_count kept, instead of counting; then the same k_insert_solid)
 //   recomputeAdjacencies    -> k_adjacency_dense (sharded: k_adjacency)
 //   buildEdges              -> unipath_stage()    (k_links, pointer-jumping list ranking, circles, edge emission, k_backfill_slots)
 //   buildHBVFromEdges       -> hbv_stage()        (end keys, radix sort, vertex ids, incidence)
@@ -21,6 +23,7 @@
 #include <cuda.h>
 
 #include "../../include/w2rap_step2.h"
+#include "../../include/w2rap_step2_counts.h"
 #include "device_reads.cuh"
 #include "count_part.cuh"
 #include "kernels.cuh"
@@ -29,6 +32,20 @@
 #include "prims.cuh"
 #include "slab_freelist.h"
 #include "places.cuh"
+
+// behind the opaque handle of w2rap_step2_count / w2rap_step2_build (include/w2rap_step2_counts.h): the k-mers one count kept and
+// what a build needs to reproduce a run's counters.  `solid` and `count` are plain cudaMallocAsync allocations on the reads' device,
+// not pieces of the device slab, which is leased per call.
+struct w2rap_counts {
+    const w2rap_device_reads* reads = nullptr;     // the read set counted: a build must pass the same handle ...
+    uint64_t n_reads = 0, n_bases = 0;              // ... still holding the same reads
+    int device = 0;
+    uint32_t min_qual = 0, f0 = 0;                  // quality floor of the count; keep floor (every k-mer seen >= f0 times is kept)
+    uint64_t n_kmer_instances = 0, n_distinct = 0, n_kept = 0;
+    uint64_t hist[101] = {};
+    ulonglong2* solid = nullptr;                    // n_kept records {w0, w1 | raw ctx}, in the order the reduce emitted them
+    uint8_t* count = nullptr;                       // n_kept counts, min(255, occurrences), parallel to `solid`
+};
 
 namespace w2r {
 
@@ -352,6 +369,9 @@ struct Pipeline {
     int world = 1, rank = 0;            // sharded run: one process per GPU, reads sharded by index, k-mers routed to owners
     ncclComm_t comm = nullptr;
 
+    bool keep_counts = false;                   // w2rap_step2_count: the reduce also writes the count of every solid record
+    const w2rap_counts* from_counts = nullptr;  // w2rap_step2_build: the solid records are selected from these instead of counted
+
     Pipeline(const DeviceReads& dr_, const w2rap_params& p_, w2rap_graph* out_, GraphOwner* ow) : dr(dr_), prm(p_), out(out_), owner(ow) {}
 
     unsigned grid(uint64_t n, unsigned block, unsigned per_sm = 16) const { return grid_for(c, n, block, per_sm); }
@@ -437,6 +457,7 @@ struct Pipeline {
     SBuf<CountSlot> cs_region;                         // two L2-resident counting regions (fallback reduce)
     SBuf<DumpRec> cs_dump;
     SBuf<ulonglong2> cs_solid; uint64_t cs_solid_cap = 0;
+    SBuf<uint8_t> cs_count;                            // keep_counts: min(255, count) of cs_solid[i], same capacity
     uint64_t cs_R = 0; uint32_t cs_logR = 0;
     bool good_done = false;
     float map_ms = 0, reduce_ms = 0, xchg_ms = 0;
@@ -544,7 +565,8 @@ struct Pipeline {
         W2R_CUDA(cudaMemsetAsync(cs_scal.p + 4, 0, 16, c.stream));
         // (a per-device attribute: set on every call — ranks driven from threads of one process each have their own device)
         const size_t stage_bytes = (size_t)2 * SKM_CHUNK * sizeof(SkmRec);
-        W2R_CUDA(cudaFuncSetAttribute(k_count_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((20u << SMEM_LOG_SLOTS_MAX) + stage_bytes)));
+        void (*const count_smem)(SmemCountParams) = keep_counts ? k_count_smem<true> : k_count_smem<false>;
+        W2R_CUDA(cudaFuncSetAttribute(count_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((20u << SMEM_LOG_SLOTS_MAX) + stage_bytes)));
         // the table_slots test hook shrinks the first table as well, so that partitions really take the fallback path
         uint32_t log1 = std::max(2u, std::min(smem_log_env, SMEM_LOG_SLOTS_MAX));
         if (prm.table_slots) log1 = (uint32_t)std::max(2, std::min((int)SMEM_LOG_SLOTS_MAX, (int)cs_logR - 6));
@@ -552,16 +574,16 @@ struct Pipeline {
         const bool two_per_sm = log1 <= 12 && !prm.table_slots;
         const uint32_t chunk1 = two_per_sm ? SKM_CHUNK / 2 : SKM_CHUNK;
         SmemCountParams sc{xrecs, xcur, runs.part_base, runs.slab_off, nslab, (uint32_t)Pown, prm.min_freq, cs_hist.p, cs_solid.p, cs_scal.p + 1, cs_solid_cap, cs_flags.p + 2,
-                           prm.dump_kmers == 2 ? cs_dump.p : nullptr, cs_scal.p + 2, failed.p, cs_scal.p + 4, log1, chunk1, nullptr, 0};
+                           prm.dump_kmers == 2 ? cs_dump.p : nullptr, cs_scal.p + 2, failed.p, cs_scal.p + 4, log1, chunk1, nullptr, 0, cs_count.p};
         kt_.begin(W2RAP_KT_REDUCE);
-        k_count_smem<<<(unsigned)std::min<uint64_t>(Pown, (uint64_t)c.sm_count * (two_per_sm ? 2 : 1)), two_per_sm ? 512 : 1024, ((size_t)20u << log1) + (size_t)2 * chunk1 * sizeof(SkmRec), c.stream>>>(sc); c.launches++; ++n_groups;
+        count_smem<<<(unsigned)std::min<uint64_t>(Pown, (uint64_t)c.sm_count * (two_per_sm ? 2 : 1)), two_per_sm ? 512 : 1024, ((size_t)20u << log1) + (size_t)2 * chunk1 * sizeof(SkmRec), c.stream>>>(sc); c.launches++; ++n_groups;
         kt_.end();
         W2R_CUDA(cudaGetLastError());
         const uint64_t nfail1 = (log1 < SMEM_LOG_SLOTS_MAX && !prm.table_slots) ? d2h_scalar(c, cs_scal.p + 4) : 0;
         if (nfail1) {
             SmemCountParams sc2 = sc;
             sc2.failed = failed2.p; sc2.failed_cursor = cs_scal.p + 5; sc2.log_slots = SMEM_LOG_SLOTS_MAX; sc2.chunk = SKM_CHUNK; sc2.plist = failed.p; sc2.nlist = (uint32_t)nfail1;
-            k_count_smem<<<(unsigned)std::min<uint64_t>(nfail1, (uint64_t)c.sm_count), 1024, ((size_t)20u << SMEM_LOG_SLOTS_MAX) + stage_bytes, c.stream>>>(sc2); c.launches++; ++n_groups;
+            count_smem<<<(unsigned)std::min<uint64_t>(nfail1, (uint64_t)c.sm_count), 1024, ((size_t)20u << SMEM_LOG_SLOTS_MAX) + stage_bytes, c.stream>>>(sc2); c.launches++; ++n_groups;
             W2R_CUDA(cudaGetLastError());
         }
         const SBuf<uint32_t>& failed_final = nfail1 ? failed2 : failed;
@@ -608,7 +630,7 @@ struct Pipeline {
                     k_count_region<<<gr, 256, 0, gs>>>(xrecs, xcur, i0, g, rv2, rp); c.launches++;
                     W2R_CUDA(cudaGetLastError());
                 }
-                ScanParams sp{greg, R, prm.min_freq, cs_hist.p, cs_solid.p, cs_scal.p + 1, cs_solid_cap, prm.dump_kmers == 2 ? cs_dump.p : nullptr, cs_scal.p + 2, flag, cs_flags.p + 2};
+                ScanParams sp{greg, R, prm.min_freq, cs_hist.p, cs_solid.p, cs_scal.p + 1, cs_solid_cap, prm.dump_kmers == 2 ? cs_dump.p : nullptr, cs_scal.p + 2, flag, cs_flags.p + 2, cs_count.p};
                 k_scan_region<<<grid(R, 256, 4), 256, 0, gs>>>(sp); c.launches++;
                 W2R_CUDA(cudaGetLastError());
             };
@@ -650,7 +672,8 @@ struct Pipeline {
                             if (d2h_scalar(c, one_flag)) ok = false;
                         }
                         if (ok) break;
-                        // roll back what the successful sub-ranges of this split emitted, then split finer
+                        // roll back what the successful sub-ranges of this split emitted, then split finer (restoring the solid cursor is
+                        // enough for cs_count too: the counts are written at the same positions as the records and get overwritten alike)
                         W2R_CUDA(cudaMemcpyAsync(cs_scal.p + 1, snapshot, 16, cudaMemcpyHostToDevice, c.stream));
                         W2R_CUDA(cudaMemcpyAsync(cs_hist.p, hist_snapshot.data(), 104 * 8, cudaMemcpyHostToDevice, c.stream));
                         W2R_CUDA(cudaStreamSynchronize(c.stream));
@@ -785,6 +808,11 @@ struct Pipeline {
                         if (solid_used) W2R_CUDA(cudaMemcpyAsync(bigger.p, cs_solid.p, solid_used * sizeof(ulonglong2), cudaMemcpyDeviceToDevice, c.stream));
                         cs_solid = std::move(bigger);
                         cs_solid_cap = cs_solid.n;
+                        if (keep_counts) {           // the parallel count array grows with it, and keeps what earlier passes wrote
+                            SBuf<uint8_t> bigger_count(c, cs_solid_cap);
+                            if (solid_used) W2R_CUDA(cudaMemcpyAsync(bigger_count.p, cs_count.p, solid_used, cudaMemcpyDeviceToDevice, c.stream));
+                            cs_count = std::move(bigger_count);
+                        }
                     }
                 }
                 trace_mark("count: solid staging");
@@ -822,7 +850,27 @@ struct Pipeline {
             W2R_CUDA(cudaStreamSynchronize(c.stream));
         }
         cs_region.release(); cs_dump.release();
-        build_dictionary(n_solid_local, n_distinct);
+        n_solid_local_ = n_solid_local; n_distinct_ = n_distinct;
+    }
+
+    // w2rap_step2_build: instead of counting, the solid records are the kept records (w2rap_step2_count) seen >= min_freq times,
+    // selected in the order the reduce emitted them (k_select_solid); the counters of the count are the run's counters
+    void select_stage() {
+        const w2rap_counts& h = *from_counts;
+        out->n_kmer_instances = h.n_kmer_instances;
+        for (int i = 0; i <= 100; ++i) out->hist[i] = h.hist[i];
+        n_distinct_ = h.n_distinct;
+        n_solid_local_ = 0;
+        cs_solid.alloc(c, h.n_kept);
+        if (!h.n_kept) return;
+        const uint64_t tiles = (h.n_kept + SCAN_TILE - 1) / SCAN_TILE;
+        SBuf<uint32_t> tile_n(c, tiles);
+        SBuf<uint64_t> tile_base(c, tiles), total(c, 1);
+        W2R_LAUNCH(c, k_select_tile_counts, (unsigned)tiles, SCAN_THREADS, 0, (const uint8_t*)h.count, h.n_kept, prm.min_freq, tile_n.p);
+        exclusive_scan<uint32_t, uint64_t>(c, tile_n.p, tiles, tile_base.p, total.p);
+        W2R_LAUNCH(c, k_select_solid, (unsigned)tiles, SCAN_THREADS, 0, (const ulonglong2*)h.solid, (const uint8_t*)h.count, h.n_kept, prm.min_freq,
+                   (const uint64_t*)tile_base.p, cs_solid.p);
+        n_solid_local_ = d2h_scalar(c, total.p);
     }
 
     // the pathing filter (kmer.cuh: PathDict): W slices of path_slice_words words, zeroed; its bits are set while the dictionary is built
@@ -844,7 +892,7 @@ struct Pipeline {
 
     // One GPU: the dictionary (kmers/ReadPather.h:176-349) as an open-addressing table over all solid k-mers.  Sharded: every rank keeps
     // the solid k-mers it counted; graph_stage_sharded() builds its local table from them.
-    uint64_t n_solid_local_ = 0;
+    uint64_t n_solid_local_ = 0, n_distinct_ = 0;     // from count_stage() or select_stage() to build_dictionary()
     uint32_t count_logP_ = 0;
     // the dictionary the reads are pathed against (kmer.cuh: PathDict)
     SBuf<PathSlice> path_slices;
@@ -1558,16 +1606,27 @@ struct Pipeline {
     }
     cudaStream_t copy_stream = nullptr;     // the graph travels to the host while the reads are pathed
 
-    void run() {
+    void begin() {
         W2R_CUDA(cudaStreamCreateWithFlags(&c.stream, cudaStreamNonBlocking));
         g_alloc_host_ms = 0;
         kt_.s = c.stream;
         c.verbose = prm.verbose != 0;
+        out->n_reads = dr.n; out->n_bases = dr.n_bases;
+    }
+
+    void run() {
+        begin();
         StageTimer total(c), st_t(c);
         total.start();
-        out->n_reads = dr.n; out->n_bases = dr.n_bases;
-        say(c, "creating kmers from reads...");
-        st_t.start(); count_stage();
+        st_t.start();
+        if (from_counts) {
+            say(c, "selecting kmers with Freq >= %u from the counts kept at Freq >= %u", prm.min_freq, from_counts->f0);
+            select_stage();
+        } else {
+            say(c, "creating kmers from reads...");
+            count_stage();
+        }
+        build_dictionary(n_solid_local_, n_distinct_);
         out->timings.count_ms = st_t.stop();
         good.release();
         if (world > 1) {
@@ -1671,13 +1730,52 @@ struct Pipeline {
         say(c, "%llu edges of total length %llu; %llu vertices", (unsigned long long)E, (unsigned long long)neb, (unsigned long long)nv);
     }
 
+    // w2rap_step2_count: the count stage alone, with the reduce keeping every k-mer seen >= f0 = prm.min_freq times and its count.
+    // The kept records and counts leave the (per-call) device slab for allocations the handle owns: 17 bytes per kept k-mer.
+    void run_count(w2rap_counts* h) {
+        begin();
+        keep_counts = true;
+        StageTimer total(c);
+        total.start();
+        say(c, "creating kmers from reads...");
+        count_stage();
+        const uint64_t n = n_solid_local_;
+        out->n_distinct = n_distinct_; out->n_solid = n;
+        say(c, "%llu kmers counted, %llu with Freq >= %u kept", (unsigned long long)n_distinct_, (unsigned long long)n, prm.min_freq);
+        const double t0 = now_ms();
+        cudaError_t e = cudaMallocAsync((void**)&h->solid, std::max<uint64_t>(n, 1) * sizeof(ulonglong2), c.stream);
+        if (e == cudaSuccess) e = cudaMallocAsync((void**)&h->count, std::max<uint64_t>(n, 1), c.stream);
+        g_alloc_host_ms += now_ms() - t0;
+        W2R_CUDA(e);
+        if (n) {
+            W2R_CUDA(cudaMemcpyAsync(h->solid, cs_solid.p, n * sizeof(ulonglong2), cudaMemcpyDeviceToDevice, c.stream));
+            W2R_CUDA(cudaMemcpyAsync(h->count, cs_count.p, n, cudaMemcpyDeviceToDevice, c.stream));
+        }
+        W2R_CUDA(cudaStreamSynchronize(c.stream));
+        cs_solid.release(); cs_count.release(); good.release();
+        h->n_kept = n; h->n_distinct = n_distinct_; h->n_kmer_instances = out->n_kmer_instances;
+        for (int i = 0; i <= 100; ++i) h->hist[i] = out->hist[i];
+        if (!dump_host.empty()) {
+            std::sort(dump_host.begin(), dump_host.end(), [](const DumpRec& a, const DumpRec& b) { return a.w0 < b.w0 || (a.w0 == b.w0 && a.w1 < b.w1); });
+            out->n_dump = dump_host.size();
+            out->dump = out_alloc<w2rap_kmer_rec>(owner, dump_host.size());
+            memcpy(out->dump, dump_host.data(), dump_host.size() * sizeof(DumpRec));
+        }
+        out->timings.count_ms = out->timings.total_ms = total.stop();
+        kt_.resolve(out->timings.kernel_ms);
+        out->timings.alloc_host_ms = (float)g_alloc_host_ms;
+        out->timings.n_records = n_records;
+        out->timings.kernel_launches = c.launches;
+        out->timings.count_launches = c.count_launches;
+    }
+
     ~Pipeline() {
         // free stream-ordered buffers before the stream goes away (and not under a transfer that still writes into them)
         if (dict_stream) cudaStreamSynchronize(dict_stream);
         if (copy_stream) { cudaStreamSynchronize(copy_stream); cudaStreamDestroy(copy_stream); }
         good.release(); solid_slots.release(); dense_slots.release(); edge_bases.release(); edge_off.release(); edge_len.release();
         edge_vertices.release(); fwd_xlat.release(); rev_xlat.release(); involution.release(); hleft.release();
-        cs_scal.release(); cs_flags.release(); cs_hist.release(); cs_region.release(); cs_dump.release(); cs_solid.release();
+        cs_scal.release(); cs_flags.release(); cs_hist.release(); cs_region.release(); cs_dump.release(); cs_solid.release(); cs_count.release();
         path_slices.release(); path_bloom.release(); hright.release(); from_e.release(); to_e.release();
         hcanon.release(); from_n.release(); to_n.release();
         if (dict_stream) { cudaStreamSynchronize(dict_stream); cudaStreamDestroy(dict_stream); cudaEventDestroy(dict_ready); }
@@ -1830,7 +1928,9 @@ static void check_params(const w2rap_params* p) {
 struct w2rap_comm { int world, rank, device; w2r::ncclComm_t comm; };
 
 namespace w2r {
-static void run_on_device(DeviceReads& dr, const w2rap_params* p, w2rap_graph* out, float h2d_ms, const w2rap_comm* cm = nullptr, double t_entry = 0) {
+// count_into: w2rap_step2_count (the count stage alone, into the handle); build_from: w2rap_step2_build (select, then the rest)
+static void run_on_device(DeviceReads& dr, const w2rap_params* p, w2rap_graph* out, float h2d_ms, const w2rap_comm* cm = nullptr, double t_entry = 0,
+                          w2rap_counts* count_into = nullptr, const w2rap_counts* build_from = nullptr) {
     GraphOwner* owner = new GraphOwner();
     memset(out, 0, sizeof(*out));
     out->_owner = owner;
@@ -1842,7 +1942,8 @@ static void run_on_device(DeviceReads& dr, const w2rap_params* p, w2rap_graph* o
         check_device(dr.device, pl.c);
         pl.c.slab = lease.slab;
         const double t_run = now_ms();
-        pl.run();
+        pl.from_counts = build_from;
+        if (count_into) pl.run_count(count_into); else pl.run();
         out->timings.h2d_ms = h2d_ms;
         out->timings.total_ms += h2d_ms;
         out->timings.host_pre_ms = t_entry ? (float)(t_run - t_entry) : 0.f;
@@ -2008,6 +2109,60 @@ int w2rap_step2_run_sharded(const w2rap_reads* shard, const w2rap_params* p, w2r
     cudaStreamSynchronize(us); d.release(); cudaStreamDestroy(us); cudaEventDestroy(e0); cudaEventDestroy(e1);
     if (comm->rank == 0 && p->workdir && p->workdir[0]) { std::string f = std::string(p->workdir) + "/small_K.freqs"; int rc = w2rap_write_freqs(f.c_str(), out, err, errlen); if (rc) return rc; }
     W2R_API_END
+}
+
+// ---- count once, build for several min_freq (include/w2rap_step2_counts.h)
+int w2rap_step2_count(w2rap_device_reads* reads, const w2rap_params* p, w2rap_counts** counts, w2rap_graph* summary, char* err, size_t errlen) {
+    W2R_API_BEGIN
+    if (!reads || !counts) W2R_FAIL(W2RAP_ERR_BAD_ARG, "null argument");
+    *counts = nullptr;
+    check_params(p);
+    if (p->dump_kmers == 1) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers 1 dumps the solid dictionary, which only a build makes: a count takes dump_kmers 0 or 2");
+    if (p->dump_kmers > 2) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers must be 0 or 2 for a count");
+    w2rap_counts* h = new w2rap_counts();
+    h->reads = reads; h->n_reads = reads->d.n; h->n_bases = reads->d.n_bases; h->device = reads->d.device;
+    h->min_qual = p->min_qual; h->f0 = p->min_freq;
+    w2rap_graph local;
+    w2rap_graph* out = summary ? summary : &local;
+    try {
+        run_on_device(reads->d, p, out, 0.f, nullptr, 0, h);
+    } catch (...) { w2rap_step2_counts_release(h); throw; }
+    int rc = W2RAP_OK;
+    if (p->workdir && p->workdir[0]) { std::string f = std::string(p->workdir) + "/small_K.freqs"; rc = w2rap_write_freqs(f.c_str(), out, err, errlen); }
+    if (!summary) w2rap_step2_free(&local);
+    if (rc) { w2rap_step2_counts_release(h); return rc; }
+    *counts = h;
+    W2R_API_END
+}
+
+int w2rap_step2_build(w2rap_device_reads* reads, const w2rap_counts* counts, const w2rap_params* p, w2rap_graph* out, char* err, size_t errlen) {
+    W2R_API_BEGIN
+    if (!reads || !counts || !out) W2R_FAIL(W2RAP_ERR_BAD_ARG, "null argument");
+    check_params(p);
+    if (p->min_freq < counts->f0)
+        W2R_FAIL(W2RAP_ERR_BAD_ARG, "min_freq %u is below the keep floor %u of these counts (k-mers seen fewer times were not kept): count again with min_freq <= %u",
+                 p->min_freq, counts->f0, p->min_freq);
+    if (p->min_qual != counts->min_qual)
+        W2R_FAIL(W2RAP_ERR_BAD_ARG, "min_qual %u differs from the min_qual %u these counts were made with (the quality floor changes the counts): count again",
+                 p->min_qual, counts->min_qual);
+    if (p->dump_kmers == 2) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers 2 (every distinct k-mer with its count) comes from w2rap_step2_count, not from a build");
+    if (p->dump_kmers > 2) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers must be 0 or 1 for a build");
+    if (reads != counts->reads || reads->d.n != counts->n_reads || reads->d.n_bases != counts->n_bases)
+        W2R_FAIL(W2RAP_ERR_BAD_ARG, "the reads handle is not the one these counts were made from: a build paths the reads that were counted");
+    run_on_device(reads->d, p, out, 0.f, nullptr, 0, nullptr, counts);
+    if (p->workdir && p->workdir[0]) { std::string f = std::string(p->workdir) + "/small_K.freqs"; int rc = w2rap_write_freqs(f.c_str(), out, err, errlen); if (rc) return rc; }
+    W2R_API_END
+}
+
+void w2rap_step2_counts_release(w2rap_counts* counts) {
+    if (!counts) return;
+    cudaSetDevice(counts->device);
+    // (stream-ordered allocations: every call that used them has drained its stream before returning)
+    if (counts->solid) cudaFreeAsync(counts->solid, 0);
+    if (counts->count) cudaFreeAsync(counts->count, 0);
+    cudaStreamSynchronize(0);
+    cudaGetLastError();
+    delete counts;
 }
 
 void* w2rap_step2_host_alloc(size_t bytes) {
