@@ -1,7 +1,7 @@
 """Runs the read-batch cases of test_upload_batches.py in a fresh process: the library reads W2RAP_UPLOAD_BATCHES (and the other
 diagnostic switches) once per process, so each switch setting needs a process of its own.
 
-usage: batch_case_runner.py hook|smem|reject
+usage: batch_case_runner.py hook|reject
 
 Every case runs the product through w2rap_step2_run twice, from the numpy buffers (pageable) and from buffers taken from
 w2rap_step2_host_alloc (pinned: only then does the copy of batch b+1 overlap the map of batch b), and compares both with the oracle
@@ -198,11 +198,6 @@ def main():
             cases.append(("tiny region", tiny_region_case))
         cases.append(("counts across batches", spread_case))
         cases += list(degenerate_cases())
-    elif mode == "smem":        # W2RAP_SMEM_LOG=10: partitions that overflow the small first table go to a second k_count_smem launch
-        rs = T.rich_set(seed=41, genome=60000, cov=50, families=4, palindromes=3, plasmid=2000, pq_mode=1, vary_len=True)
-        want = oracle(rs, dump_kmers=2, apply_fixpaths=1)
-        cases.append(("rich, second shared-memory table", lambda: check("rich, second shared-memory table", rs, want, check_passes=lambda g: g >= 2,
-                                                                         dump_kmers=2, apply_fixpaths=1)))
     else:
         raise SystemExit("unknown mode " + mode)
     failed = 0

@@ -9,7 +9,6 @@ import os
 import re
 import shutil
 import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -191,26 +190,6 @@ def test_reduce_paths_keep_counts(case):
             assert_build_matches(s, rs, ch, "%s min_freq=%d" % (case, mf), min_freq=mf, dump_kmers=1, **kw)
     finally:
         s.close()
-
-
-def _smem_log_child():
-    """(in a child process with W2RAP_SMEM_LOG=10: two 512-thread CTAs per SM with half-size staging, then the 8192-slot table)"""
-    rs = T.rich_set(seed=21, genome=100000, cov=60, families=4, palindromes=2, plasmid=1500)
-    s = Session(rs)
-    try:
-        ch, _ = s.count(min_freq=3)
-        for mf in (3, 4):
-            assert_build_matches(s, rs, ch, "W2RAP_SMEM_LOG=10 min_freq=%d" % mf, min_freq=mf, dump_kmers=1, apply_fixpaths=1)
-    finally:
-        s.close()
-    print("OK")
-
-
-@pytest.mark.gpu
-def test_small_shared_memory_table_keeps_counts():
-    env = dict(os.environ, W2RAP_SMEM_LOG="10", PYTHONPATH=HERE)
-    r = subprocess.run([sys.executable, "-c", "import test_count_once as M; M._smem_log_child()"], env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0 and "OK" in r.stdout, (r.stdout[-3000:], r.stderr[-3000:])
 
 
 @pytest.mark.gpu

@@ -56,13 +56,12 @@ def test_long_reads_span_several_map_tiles(T):
     assert int(rs.len.max()) > 500 and got["n_pathed"] > 0
 
 
-@pytest.mark.parametrize("fine_recs,smem_log", [("300000", "13"), ("4000000", "13"), ("24000", "10")])
-def test_partitions_that_do_not_fit_shared_memory(fine_recs, smem_log):
+@pytest.mark.parametrize("fine_recs", ["300000", "4000000"])
+def test_partitions_that_do_not_fit_shared_memory(fine_recs):
     """Oversized partitions: every partition fails the shared-memory count and goes through the L2 region in bulk groups
-    (300 k records each), one partition larger than the region itself is split into hash sub-ranges (4 M), and a small first
-    table (1024 slots) hands most partitions to the second, larger one."""
+    (300 k records each), and one partition larger than the region itself is split into hash sub-ranges (4 M)."""
     here = os.path.dirname(os.path.abspath(__file__))
-    env = dict(os.environ, W2RAP_FINE_RECS=fine_recs, W2RAP_SMEM_LOG=smem_log, PYTHONPATH=here)
+    env = dict(os.environ, W2RAP_FINE_RECS=fine_recs, PYTHONPATH=here)
     r = subprocess.run([sys.executable, os.path.join(here, "env_case_runner.py"), "100000", "60", "21"], env=env, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "OK" in r.stdout, (r.stdout[-2000:], r.stderr[-2000:])
     passes = int(r.stdout.split("passes=")[1].split()[0])

@@ -17,8 +17,8 @@ pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def run_child(mode, batches, timeout=900, **env):
-    e = dict(os.environ, W2RAP_UPLOAD_BATCHES=str(batches), PYTHONPATH=HERE, **env)
+def run_child(mode, batches, timeout=900):
+    e = dict(os.environ, W2RAP_UPLOAD_BATCHES=str(batches), PYTHONPATH=HERE)
     return subprocess.run([sys.executable, os.path.join(HERE, "batch_case_runner.py"), mode], env=e, capture_output=True, text=True, timeout=timeout)
 
 
@@ -30,13 +30,6 @@ def test_batched_runs_match_the_oracle(batches):
     r = run_child("hook", batches)
     assert r.returncode == 0 and "FAIL" not in r.stdout, (r.stdout[-6000:], r.stderr[-3000:])
     assert r.stdout.count("OK ") == (9 if batches == 8 else 8), r.stdout
-
-
-def test_second_shared_memory_table_with_several_runs():
-    """W2RAP_SMEM_LOG=10: the partitions that overflow the 1024-slot table are counted by a second k_count_smem launch over the
-    list of failed partitions, here with 3 runs each."""
-    r = run_child("smem", 3, W2RAP_SMEM_LOG="10")
-    assert r.returncode == 0 and "OK " in r.stdout, (r.stdout[-6000:], r.stderr[-3000:])
 
 
 @pytest.mark.parametrize("value", ["0", "17", "eight"])

@@ -33,6 +33,7 @@ namespace w2r {
 constexpr uint32_t MINI_TILE = 192;                       // k-mers per tile (a 250-base read is one tile)
 constexpr uint32_t MINI_NU = 8;                           // hashes per lane: positions 32u + lane, u < 8, cover the 192 + 45 m-mers of a tile
 constexpr uint32_t MAP_CHUNK = 512;                       // records a warp reserves at a time in the staging area (>= MINI_TILE)
+constexpr uint32_t MAP_CTAS_PER_SM = 6;                   // k_minimizer_map's occupancy: its register cap, its grid, the staging allowance
 struct MiniParams {
     uint32_t logP, npass, pass;
     uint32_t* count;                 // records per partition (this read batch)
@@ -47,7 +48,7 @@ struct MiniParams {
 // and k-mers per partition.  After an exclusive scan of the counts, launch 2 (k_scatter_records: a copy kernel) moves every record
 // to its partition.  Exact sizes mean no capacity guess per partition can overflow, whatever the multiplicity skew of the read set
 // (a repeat with 10^4 copies just makes its partitions long).
-__global__ void __launch_bounds__(256, 6) k_minimizer_map(ReadsView r, uint64_t first, uint64_t count, const uint16_t* __restrict__ good, MiniParams mp) {
+__global__ void __launch_bounds__(256, MAP_CTAS_PER_SM) k_minimizer_map(ReadsView r, uint64_t first, uint64_t count, const uint16_t* __restrict__ good, MiniParams mp) {
     __shared__ uint32_t wbuf[8][MINI_TILE];
     __shared__ uint32_t sbuf[8][MINI_TILE];               // segment list of the tile: start | n << 16
     uint32_t* wb = wbuf[threadIdx.x >> 5];
@@ -235,12 +236,12 @@ __global__ void __launch_bounds__(256) k_count_region(const SkmRec* __restrict__
 // With ~2^18 partitions a partition holds ~20 k k-mer instances and a few thousand distinct k-mers: one CTA counts it in a
 // shared-memory table, so the per-instance atomics are shared-memory atomics instead of L2 atomics (the L2-resident region count
 // is limited by L2 atomic throughput, about one k-mer per 30 ps chip-wide).  Partitions whose distinct k-mers do not fit are listed
-// in `failed`: they are retried with a larger table and, failing that, go through the region path.
+// in `failed` and go through the region path.
 constexpr uint32_t SMEM_LOG_SLOTS_MAX = 13;                    // 8192 slots: 128 KB keys + 32 KB count|ctx = 160 KB
 constexpr uint32_t SMEM_MAX_PROBE = 512;
 constexpr uint32_t COUNT_STOP = 1u << 16;                      // counters stop here (>= 255 is all anyone asks); + one add per racing thread
 constexpr uint32_t SMEM_MAX_BATCH = 16;                        // runs (read batches / source ranks) that make up one partition
-constexpr uint32_t SKM_CHUNK = 1024;                           // most records per staging buffer (32 KB), two buffers
+constexpr uint32_t SKM_CHUNK = 1024;                           // records per staging buffer (32 KB), two buffers
 struct SmemCountParams {
     const SkmRec* recs;
     const uint32_t* cursor;         // [nbatch][P] records of partition p in slab bi
@@ -252,10 +253,8 @@ struct SmemCountParams {
     unsigned long long* hist;       // [104]
     ulonglong2* solid_out; unsigned long long* solid_cursor; uint64_t solid_cap; int* solid_overflow;
     DumpRec* dump_out; unsigned long long* dump_cursor;
-    uint32_t* failed; unsigned long long* failed_cursor;       // partitions that did not fit this table size
-    uint32_t log_slots;                                        // table size of this launch
-    uint32_t chunk;                                            // records per staging buffer (two buffers); <= SKM_CHUNK
-    const uint32_t* plist; uint32_t nlist;                     // if set: only these partitions (the ones a smaller table could not hold)
+    uint32_t* failed; unsigned long long* failed_cursor;       // partitions that did not fit the table
+    uint32_t log_slots;                                        // log2 of the table's slots: SMEM_LOG_SLOTS_MAX, less under the table_slots test hook
     uint8_t* count_out;                                        // k_count_smem<true>: min(255, count) of solid_out[i] at count_out[i]
 };
 
@@ -315,8 +314,7 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
     const uint32_t SMEM_SLOTS = 1u << sp.log_slots;
     ulonglong2* keys = reinterpret_cast<ulonglong2*>(smem_raw);             // {w0, w1}; empty = all ones (a canonical 60-mer never starts with 32 T's)
     uint32_t* ccs = reinterpret_cast<uint32_t*>(keys + SMEM_SLOTS);         // count (low 24 bits) | ctx << 24
-    SkmRec* stage = reinterpret_cast<SkmRec*>(smem_raw + (size_t)20 * SMEM_SLOTS);   // [2][sp.chunk]
-    const uint32_t CHUNK = sp.chunk;
+    SkmRec* stage = reinterpret_cast<SkmRec*>(smem_raw + (size_t)20 * SMEM_SLOTS);   // [2][SKM_CHUNK]
     __shared__ __align__(8) uint64_t mbar[2];
     __shared__ unsigned int sh_hist[104];
     __shared__ int sh_fail;
@@ -328,24 +326,22 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
     for (int j = threadIdx.x; j < 104; j += blockDim.x) sh_hist[j] = 0;
     if (threadIdx.x == 0) { mbar_init(&mbar[0], 1); mbar_init(&mbar[1], 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
     __syncthreads();
-    const uint32_t n_todo = sp.plist ? sp.nlist : sp.P;
     // Warp 0 stages the records: lane bi owns run bi of a partition (a read batch / source rank).  The run descriptors of the NEXT
     // partition are loaded a whole partition ahead and sit in registers, so that issuing a chunk is a few shuffles and one bulk copy
     // per lane (one thread walking the runs with dependent global loads made warp 0 late at every chunk barrier: ~20 % of the
     // kernel's stall samples).
     uint32_t cu_cnt = 0, nx_cnt = 0;                             // records of my run in the current / next partition
     const SkmRec* cu_src = nullptr; const SkmRec* nx_src = nullptr;
-    auto load_desc = [&](uint32_t pi, uint32_t& cnt, const SkmRec*& src) {
+    auto load_desc = [&](uint32_t p, uint32_t& cnt, const SkmRec*& src) {
         cnt = 0; src = nullptr;
-        if (pi < n_todo && lane < sp.nbatch) {
-            const uint32_t p = sp.plist ? sp.plist[pi] : pi;
+        if (p < sp.P && lane < sp.nbatch) {
             cnt = sp.cursor[(uint64_t)lane * sp.P + p];
             src = sp.recs + sp.batch_off[lane] + sp.part_base[(uint64_t)lane * sp.P + p];
         }
     };
     // all lanes of warp 0: stage chunk c of the partition described by (cnt, src) into buffer bf
     auto issue = [&](uint32_t cnt, const SkmRec* src, uint32_t c, uint32_t bf) {
-        const uint32_t lo = c * CHUNK, hi = lo + CHUNK;
+        const uint32_t lo = c * SKM_CHUNK, hi = lo + SKM_CHUNK;
         uint32_t incl = cnt;
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, d); if ((int)lane >= d) incl += t; }
@@ -353,7 +349,7 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
         const uint32_t s = acc > lo ? acc : lo, e = acc + cnt < hi ? acc + cnt : hi;
         if (s < e) {
             mbar_expect_tx(&mbar[bf], (e - s) * (uint32_t)sizeof(SkmRec));
-            bulk_g2s(stage + (size_t)bf * CHUNK + (s - lo), src + (s - acc), (e - s) * (uint32_t)sizeof(SkmRec), &mbar[bf]);
+            bulk_g2s(stage + (size_t)bf * SKM_CHUNK + (s - lo), src + (s - acc), (e - s) * (uint32_t)sizeof(SkmRec), &mbar[bf]);
         }
         __syncwarp();                                            // every expect_tx precedes the arrival
         if (lane == 0) {
@@ -366,10 +362,9 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
     if (warp == 0) {
         load_desc(blockIdx.x, cu_cnt, cu_src);
         load_desc(blockIdx.x + gridDim.x, nx_cnt, nx_src);
-        if (blockIdx.x < n_todo) issue(cu_cnt, cu_src, 0, 0);
+        if (blockIdx.x < sp.P) issue(cu_cnt, cu_src, 0, 0);
     }
-    for (uint32_t pi = blockIdx.x; pi < n_todo; pi += gridDim.x) {
-        const uint32_t p = sp.plist ? sp.plist[pi] : pi;
+    for (uint32_t p = blockIdx.x; p < sp.P; p += gridDim.x) {
         {   // empty table (16-byte stores)
             const ulonglong2 ff = make_ulonglong2(~0ull, ~0ull);
             for (uint32_t j = threadIdx.x; j < SMEM_SLOTS; j += blockDim.x) keys[j] = ff;
@@ -404,17 +399,17 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
             const uint32_t bf = it & 1u;
             mbar_wait(&mbar[bf], (it >> 1) & 1u);
             const uint32_t tot = sh_tot[bf], cnt = sh_cnt[bf];
-            const bool more = (uint64_t)(c + 1) * CHUNK < tot;
+            const bool more = (uint64_t)(c + 1) * SKM_CHUNK < tot;
             // the other buffer is free: everyone left it at the barrier that ended the previous chunk
             if (warp == 0) {
                 if (more) issue(cu_cnt, cu_src, c + 1, bf ^ 1u);
                 else {
-                    if (pi + gridDim.x < n_todo) issue(nx_cnt, nx_src, 0, bf ^ 1u);
+                    if (p + gridDim.x < sp.P) issue(nx_cnt, nx_src, 0, bf ^ 1u);
                     cu_cnt = nx_cnt; cu_src = nx_src;
-                    load_desc(pi + 2 * gridDim.x, nx_cnt, nx_src);   // (in flight while this chunk and the next partition are counted)
+                    load_desc(p + 2 * gridDim.x, nx_cnt, nx_src);   // (in flight while this chunk and the next partition are counted)
                 }
             }
-            const SkmRec* st = stage + (size_t)bf * CHUNK;
+            const SkmRec* st = stage + (size_t)bf * SKM_CHUNK;
             // Every warp takes an equal share of the chunk's records, in groups of <= 32 (a fixed deal of 32-record groups left most
             // warps idle in a partition's short last chunk: 24 % of all stall samples sat at the barrier below).  Inside a group the
             // k-mers are numbered consecutively across the records and lane l takes k-mer t + l.  Which record that is: the records that
@@ -454,8 +449,8 @@ __global__ void __launch_bounds__(1024, 1) k_count_smem(SmemCountParams sp) {
         // buffer this partition's last chunk came through (buffer (it - 1) & 1): the barrier above was the last read of it, the
         // bulk copy into it has completed (waited on), and the next partition's chunk 0 is already in flight into the OTHER buffer.
         // Nothing is issued into this one before the next partition's first chunk has been waited for, which is after the barrier
-        // that ends this partition.  It holds CHUNK * 32 >= 16 KB; the counts take SMEM_SLOTS <= 8 KB.
-        uint8_t* kept = reinterpret_cast<uint8_t*>(stage + (size_t)((it - 1u) & 1u) * CHUNK);
+        // that ends this partition.  It holds SKM_CHUNK * 32 = 32 KB; the counts take SMEM_SLOTS <= 8 KB.
+        uint8_t* kept = reinterpret_cast<uint8_t*>(stage + (size_t)((it - 1u) & 1u) * SKM_CHUNK);
         const bool failed = sh_fail != 0;
         if (failed) {
             if (threadIdx.x == 0) sp.failed[atomicAdd(sp.failed_cursor, 1ull)] = p;

@@ -456,10 +456,10 @@ struct alignas(8) PathMeta { uint32_t x, y; };   // x = first id in the staging 
 // and the requester gets the 32-bit candidate mask.  Each requester then looks up its own first candidate in the dictionary
 // (all requesters at once), and continues along its read.
 constexpr int PATH_GAP_BATCH = 4;
-template <int MIN_CTAS>
-__global__ void __launch_bounds__(128, MIN_CTAS) k_path_reads(ReadsView r, GraphView g, const uint32_t* __restrict__ list, uint64_t n_rows,
-                                                    int32_t* __restrict__ stage, uint32_t cap, uint32_t left_cap, int32_t* __restrict__ out_offset,
-                                                    PathMeta* __restrict__ out_meta, uint32_t apply_fixpaths) {
+constexpr uint32_t PATH_CTAS_PER_SM = 8;          // k_path_reads' register cap and grid (path_stage: why 8)
+__global__ void __launch_bounds__(128, PATH_CTAS_PER_SM) k_path_reads(ReadsView r, GraphView g, const uint32_t* __restrict__ list, uint64_t n_rows,
+                                                                      int32_t* __restrict__ stage, uint32_t cap, uint32_t left_cap, int32_t* __restrict__ out_offset,
+                                                                      PathMeta* __restrict__ out_meta, uint32_t apply_fixpaths) {
     // walker state in shared memory, one slot per thread, padded to an odd number of words (no bank conflicts across lanes)
     struct Slot { PathState st; uint32_t pad[(sizeof(PathState) / 4) % 2 == 0 ? 1 : 2]; };
     __shared__ Slot slots[128];

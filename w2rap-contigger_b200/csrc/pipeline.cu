@@ -451,7 +451,7 @@ struct Pipeline {
         SBuf<uint64_t> xbase, xtot, xktot;
         SBuf<unsigned long long> xoff;                 // [world + 1]
     };
-    SBuf<unsigned long long> cs_scal;                  // [0] k-mer instances, [1] solid cursor, [2] dump cursor, [4], [5] failed-partition cursors
+    SBuf<unsigned long long> cs_scal;                  // [0] k-mer instances, [1] solid cursor, [2] dump cursor, [4] failed-partition cursor
     SBuf<int> cs_flags;                                // [0] malformed quality vector, [1] record buffer overflow, [2] solid staging overflow
     SBuf<unsigned long long> cs_hist;
     SBuf<CountSlot> cs_region;                         // two L2-resident counting regions (fallback reduce)
@@ -469,12 +469,8 @@ struct Pipeline {
         if (bt.count) W2R_TIMED(W2RAP_KT_GOOD_LEN, W2R_LAUNCH(c, k_good_len, grid(bt.count, 128), 128, 0, dr.view(), bt.first, bt.count, prm.min_qual, good.p, cs_scal.p, cs_flags.p));
     }
 
-    static unsigned map_ctas() {
-        static const unsigned n = getenv("W2RAP_MAP_CTAS") ? (unsigned)atoi(getenv("W2RAP_MAP_CTAS")) : 6u;
-        return n;
-    }
     // warps of the map launch over `count` reads that take a staging chunk: each ends the launch holding one partly used chunk
-    uint64_t map_chunk_warps(uint64_t count) const { return std::min<uint64_t>(count, (uint64_t)grid(count * 32, 256, map_ctas()) * 8); }
+    uint64_t map_chunk_warps(uint64_t count) const { return std::min<uint64_t>(count, (uint64_t)grid(count * 32, 256, MAP_CTAS_PER_SM) * 8); }
 
     // map: per read batch  quality floor -> counting launch -> scan -> store launch (all queued without a host round trip, so a
     // batch is mapped as soon as it has crossed PCIe).  Returns false if the record area was too small (need = exact size).
@@ -501,7 +497,7 @@ struct Pipeline {
             W2R_CUDA(cudaEventCreate(&ev[2 * bi])); W2R_CUDA(cudaEventCreate(&ev[2 * bi + 1]));
             W2R_CUDA(cudaEventRecord(ev[2 * bi], c.stream));
             W2R_LAUNCH(c, k_copy_scalar, 1, 1, 0, (const unsigned long long*)cb.tmp_cursor.p, cb.tmp_range.p + bi);
-            if (bt.count && pl.n_inst_local) W2R_TIMED(W2RAP_KT_MAP, W2R_LAUNCH(c, k_minimizer_map, grid(bt.count * 32, 256, map_ctas()), 256, 0, rv, bt.first, bt.count, good.p, mp));
+            if (bt.count && pl.n_inst_local) W2R_TIMED(W2RAP_KT_MAP, W2R_LAUNCH(c, k_minimizer_map, grid(bt.count * 32, 256, MAP_CTAS_PER_SM), 256, 0, rv, bt.first, bt.count, good.p, mp));
             W2R_LAUNCH(c, k_copy_scalar, 1, 1, 0, (const unsigned long long*)cb.tmp_cursor.p, cb.tmp_range.p + bi + 1);
             exclusive_scan<uint32_t, uint64_t>(c, cb.part_count.p + bi * P, P, cb.part_base.p + bi * P, cb.batch_total.p + bi);
             W2R_LAUNCH(c, k_next_batch_off, 1, 1, 0, cb.batch_off.p + bi, cb.batch_total.p + bi);
@@ -556,42 +552,29 @@ struct Pipeline {
 
     // reduce: what this rank counts is `nslab` runs per owned partition (read batches on one GPU, source ranks when sharded)
     void reduce_records(const CountPlan& pl, const SkmRec* xrecs, const uint32_t* xcur, const uint32_t* xkcur, RunView runs, cudaStream_t s2, cudaEvent_t ev_fork, cudaEvent_t ev_join) {
-        static const uint32_t smem_log_env = getenv("W2RAP_SMEM_LOG") ? (uint32_t)atoi(getenv("W2RAP_SMEM_LOG")) : 13u;
         const uint64_t Pown = pl.Pown, R = cs_R;
         const uint32_t nslab = pl.nslab;
         EventTimer kt(c.stream);
         kt.start();
-        SBuf<uint32_t> failed(c, Pown), failed2(c, Pown);
-        W2R_CUDA(cudaMemsetAsync(cs_scal.p + 4, 0, 16, c.stream));
+        SBuf<uint32_t> failed(c, Pown);
+        W2R_CUDA(cudaMemsetAsync(cs_scal.p + 4, 0, 8, c.stream));
         // (a per-device attribute: set on every call — ranks driven from threads of one process each have their own device)
         const size_t stage_bytes = (size_t)2 * SKM_CHUNK * sizeof(SkmRec);
         void (*const count_smem)(SmemCountParams) = keep_counts ? k_count_smem<true> : k_count_smem<false>;
         W2R_CUDA(cudaFuncSetAttribute(count_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((20u << SMEM_LOG_SLOTS_MAX) + stage_bytes)));
-        // the table_slots test hook shrinks the first table as well, so that partitions really take the fallback path
-        uint32_t log1 = std::max(2u, std::min(smem_log_env, SMEM_LOG_SLOTS_MAX));
-        if (prm.table_slots) log1 = (uint32_t)std::max(2, std::min((int)SMEM_LOG_SLOTS_MAX, (int)cs_logR - 6));
-        // small first table (<= 4096 slots): two CTAs of 512 threads per SM, each with half-size staging buffers
-        const bool two_per_sm = log1 <= 12 && !prm.table_slots;
-        const uint32_t chunk1 = two_per_sm ? SKM_CHUNK / 2 : SKM_CHUNK;
+        // the table_slots test hook shrinks the shared-memory table as well, so that partitions really take the fallback path
+        const uint32_t log_slots = prm.table_slots ? (uint32_t)std::max(2, std::min((int)SMEM_LOG_SLOTS_MAX, (int)cs_logR - 6)) : SMEM_LOG_SLOTS_MAX;
         SmemCountParams sc{xrecs, xcur, runs.part_base, runs.slab_off, nslab, (uint32_t)Pown, prm.min_freq, cs_hist.p, cs_solid.p, cs_scal.p + 1, cs_solid_cap, cs_flags.p + 2,
-                           prm.dump_kmers == 2 ? cs_dump.p : nullptr, cs_scal.p + 2, failed.p, cs_scal.p + 4, log1, chunk1, nullptr, 0, cs_count.p};
+                           prm.dump_kmers == 2 ? cs_dump.p : nullptr, cs_scal.p + 2, failed.p, cs_scal.p + 4, log_slots, cs_count.p};
         kt_.begin(W2RAP_KT_REDUCE);
-        count_smem<<<(unsigned)std::min<uint64_t>(Pown, (uint64_t)c.sm_count * (two_per_sm ? 2 : 1)), two_per_sm ? 512 : 1024, ((size_t)20u << log1) + (size_t)2 * chunk1 * sizeof(SkmRec), c.stream>>>(sc); c.launches++; ++n_groups;
+        count_smem<<<(unsigned)std::min<uint64_t>(Pown, (uint64_t)c.sm_count), 1024, ((size_t)20u << log_slots) + stage_bytes, c.stream>>>(sc); c.launches++; ++n_groups;
         kt_.end();
         W2R_CUDA(cudaGetLastError());
-        const uint64_t nfail1 = (log1 < SMEM_LOG_SLOTS_MAX && !prm.table_slots) ? d2h_scalar(c, cs_scal.p + 4) : 0;
-        if (nfail1) {
-            SmemCountParams sc2 = sc;
-            sc2.failed = failed2.p; sc2.failed_cursor = cs_scal.p + 5; sc2.log_slots = SMEM_LOG_SLOTS_MAX; sc2.chunk = SKM_CHUNK; sc2.plist = failed.p; sc2.nlist = (uint32_t)nfail1;
-            count_smem<<<(unsigned)std::min<uint64_t>(nfail1, (uint64_t)c.sm_count), 1024, ((size_t)20u << SMEM_LOG_SLOTS_MAX) + stage_bytes, c.stream>>>(sc2); c.launches++; ++n_groups;
-            W2R_CUDA(cudaGetLastError());
-        }
-        const SBuf<uint32_t>& failed_final = nfail1 ? failed2 : failed;
-        const uint64_t nfail = d2h_scalar(c, nfail1 ? cs_scal.p + 5 : cs_scal.p + 4);
+        const uint64_t nfail = d2h_scalar(c, cs_scal.p + 4);
         if (nfail) {
             say(c, "%llu of %llu k-mer partitions did not fit shared memory; counting them through the L2 region", (unsigned long long)nfail, (unsigned long long)Pown);
             std::vector<uint32_t> fl(nfail);
-            W2R_CUDA(cudaMemcpyAsync(fl.data(), failed_final.p, nfail * 4, cudaMemcpyDeviceToHost, c.stream));
+            W2R_CUDA(cudaMemcpyAsync(fl.data(), failed.p, nfail * 4, cudaMemcpyDeviceToHost, c.stream));
             // per owned partition: largest run in records (sizes the grid) and k-mer instances (bounds its distinct k-mers)
             std::vector<uint32_t> raw((size_t)nslab * Pown), rawk((size_t)nslab * Pown);
             W2R_CUDA(cudaMemcpyAsync(raw.data(), xcur, raw.size() * 4, cudaMemcpyDeviceToHost, c.stream));
@@ -625,7 +608,7 @@ struct Pipeline {
                 if (mxg) {
                     RegionParams rp{greg, cs_logR, sub_mask, sub_id, flag};
                     RunView rv2 = runs;
-                    rv2.plist = failed_final.p;
+                    rv2.plist = failed.p;
                     dim3 gr(std::max(1u, std::min<unsigned>((mxg + 7) / 8, (unsigned)(c.sm_count * 8 / std::max(1u, std::min(g * nslab, 8u))))), g * nslab);
                     k_count_region<<<gr, 256, 0, gs>>>(xrecs, xcur, i0, g, rv2, rp); c.launches++;
                     W2R_CUDA(cudaGetLastError());
@@ -877,14 +860,12 @@ struct Pipeline {
     void alloc_path_filter(uint64_t n_solid) {
         path_slice_words = 0;
         path_bloom.release();
-        if (n_solid < 4096 || getenv("W2RAP_NO_BLOOM") || !prm.want_paths) return;
+        if (n_solid < 4096 || !prm.want_paths) return;
         // ~1.5 bytes per key (false positives ~4 %), at least 4 KB, at most 192 MB unless the dictionary is so large that a capped
         // filter would pass everything (measured at 1.44 G keys with 192 MB: every screened position probed the dictionary)
-        static const uint64_t bloom_mb = getenv("W2RAP_BLOOM_MB") ? (uint64_t)atoi(getenv("W2RAP_BLOOM_MB")) : 192;
-        const uint64_t cap = std::max<uint64_t>(bloom_mb << 20, std::min<uint64_t>(n_solid + n_solid / 2, 8ull << 30));
-        uint64_t bytes = std::min<uint64_t>(cap, std::max<uint64_t>(4096, n_solid * 2));
-        static const uint64_t exact_mb = getenv("W2RAP_BLOOM_EXACT_MB") ? (uint64_t)atoi(getenv("W2RAP_BLOOM_EXACT_MB")) : 0;      // (diagnostic sweep)
-        if (exact_mb) bytes = exact_mb << 20;
+        constexpr uint64_t PATH_FILTER_CAP = 192ull << 20;
+        const uint64_t cap = std::max<uint64_t>(PATH_FILTER_CAP, std::min<uint64_t>(n_solid + n_solid / 2, 8ull << 30));
+        const uint64_t bytes = std::min<uint64_t>(cap, std::max<uint64_t>(4096, n_solid * 2));
         path_slice_words = (uint32_t)std::max<uint64_t>(64, bytes / 4 / world);
         path_bloom.alloc(c, (size_t)path_slice_words * world);
         path_bloom.zero();
@@ -1440,8 +1421,6 @@ struct Pipeline {
         GraphView g{dict, edge_bases.p, edge_off.p, edge_len.p, fwd_xlat.p, rev_xlat.p, hcanon.p, hleft.p, hright.p, from_e.p, to_e.p, from_n.p, to_n.p};
         const ReadsView rv = dr.view();
         const unsigned block = 128;
-        static const int path_occ_grid = getenv("W2RAP_PATH_OCC") ? std::max(6, atoi(getenv("W2RAP_PATH_OCC"))) : 8;
-        const unsigned gr = grid(n, block, path_occ_grid);
         const uint32_t cap = 24, left_cap = 8;
         SBuf<int32_t> stage(c, n * cap), row_off(c, n);
         SBuf<PathMeta> meta(c, n);
@@ -1450,16 +1429,7 @@ struct Pipeline {
         // resident CTAs per SM the compiler must allow for (register cap): the kernel waits on dependent DRAM fetches, so warps in flight matter
         // measured (config 2, path stage): 8 CTAs/SM (64 registers) 96 ms, 10: 105 ms, 12 (40 registers, more spills) 81.5 ms, 14/16: 86 ms
         // round 2 (walker state in shared memory, ~350 B less stack): 12 CTAs/SM 71.8 ms, 10: 59.8 ms, 8 (64 registers): 54.9 ms
-        static const int path_occ = getenv("W2RAP_PATH_OCC") ? atoi(getenv("W2RAP_PATH_OCC")) : 8;
-        auto launch_path = [&](unsigned grd, const uint32_t* list, uint64_t rows, int32_t* stg, uint32_t cp, uint32_t lcp, int32_t* roff, PathMeta* mt) {
-            if (path_occ >= 16) W2R_LAUNCH(c, k_path_reads<16>, grd, block, 0, rv, g, list, rows, stg, cp, lcp, roff, mt, prm.apply_fixpaths);
-            else if (path_occ >= 14) W2R_LAUNCH(c, k_path_reads<14>, grd, block, 0, rv, g, list, rows, stg, cp, lcp, roff, mt, prm.apply_fixpaths);
-            else if (path_occ >= 12) W2R_LAUNCH(c, k_path_reads<12>, grd, block, 0, rv, g, list, rows, stg, cp, lcp, roff, mt, prm.apply_fixpaths);
-            else if (path_occ >= 10) W2R_LAUNCH(c, k_path_reads<10>, grd, block, 0, rv, g, list, rows, stg, cp, lcp, roff, mt, prm.apply_fixpaths);
-            else if (path_occ >= 8) W2R_LAUNCH(c, k_path_reads<8>, grd, block, 0, rv, g, list, rows, stg, cp, lcp, roff, mt, prm.apply_fixpaths);
-            else W2R_LAUNCH(c, k_path_reads<6>, grd, block, 0, rv, g, list, rows, stg, cp, lcp, roff, mt, prm.apply_fixpaths);
-        };
-        W2R_TIMED(W2RAP_KT_PATH_READS, launch_path(gr, nullptr, n, stage.p, cap, left_cap, row_off.p, meta.p));
+        W2R_TIMED(W2RAP_KT_PATH_READS, W2R_LAUNCH(c, k_path_reads, grid(n, block, PATH_CTAS_PER_SM), block, 0, rv, g, nullptr, n, stage.p, cap, left_cap, row_off.p, meta.p, prm.apply_fixpaths));
         W2R_LAUNCH(c, k_path_lens, grid(n, 256), 256, 0, meta.p, (const uint32_t*)nullptr, n, lens.p, counters.p);
         unsigned long long cnt[3];
         W2R_CUDA(cudaMemcpyAsync(cnt, counters.p, 24, cudaMemcpyDeviceToHost, c.stream));
@@ -1473,7 +1443,8 @@ struct Pipeline {
         if (n_ovf) {
             W2R_CUDA(cudaMemsetAsync(counters.p + 3, 0, 8, c.stream));
             W2R_LAUNCH(c, k_collect_overflow, grid(n, 256), 256, 0, meta.p, n, olist.p, counters.p + 3);
-            W2R_TIMED(W2RAP_KT_PATH_READS, launch_path(grid(n_ovf, block, path_occ_grid), olist.p, n_ovf, stage2.p, cap2, left2, row_off2.p, meta2.p));
+            W2R_TIMED(W2RAP_KT_PATH_READS, W2R_LAUNCH(c, k_path_reads, grid(n_ovf, block, PATH_CTAS_PER_SM), block, 0, rv, g, (const uint32_t*)olist.p, n_ovf, stage2.p, cap2, left2,
+                                                      row_off2.p, meta2.p, prm.apply_fixpaths));
             W2R_CUDA(cudaMemsetAsync(counters.p + 2, 0, 8, c.stream));
             W2R_LAUNCH(c, k_path_lens, grid(n_ovf, 256), 256, 0, meta2.p, (const uint32_t*)olist.p, n_ovf, lens.p, counters.p);
             W2R_CUDA(cudaMemcpyAsync(cnt, counters.p, 24, cudaMemcpyDeviceToHost, c.stream));
