@@ -9,6 +9,7 @@
 //                     bvec: u32 size + ceil(size/4) bytes, feudal/FieldVec.h:595-597).  to_ is rebuilt on read.
 //   .small_K.paths  : paths/long/ReadPath.cc:6-20: u64 n; per read i32 offset, u16 len, len x i32.
 //   small_K.freqs   : "i, count" lines for i = 1..100 (paths/long/BuildReadQGraph.cc:1108-1112).
+//   .small_K.gfa    : GFA 1.0 of the graph with per-edge k-mer coverage (include/w2rap_coverage.h).
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -18,7 +19,7 @@
 #include <string>
 #include <vector>
 
-#include "../../include/w2rap_step2.h"
+#include "../../include/w2rap_coverage.h"
 
 namespace {
 
@@ -208,6 +209,69 @@ int w2rap_write_hbv(const char* path, const w2rap_graph* g, char* err, size_t er
             ok = ok && f.put(rc.data(), nb);
         }
     }
+    if (!ok) return fail(W2RAP_ERR_IO, err, errlen, "short write to %s", path);
+    return W2RAP_OK;
+}
+
+// include/w2rap_coverage.h: segments are canonical edges named by their fwd hbv id; links are pairs of hbv edges meeting at a vertex,
+// each written once for itself and its complement.
+int w2rap_write_gfa(const char* path, const w2rap_graph* g, const w2rap_seq_cov* edge_cov, char* err, size_t errlen) {
+    if (!path || !g) return fail(W2RAP_ERR_BAD_ARG, err, errlen, "%s", "null argument");
+    const uint64_t E = g->n_edges, nv = g->n_vertices, nh = g->n_hbv_edges;
+    if (E && (!g->edge_vertices || !g->fwd_xlat || !g->involution))
+        return fail(W2RAP_ERR_BAD_ARG, err, errlen, "%s", "graph without edge_vertices, fwd_xlat or involution (a non-root result of a graph_on_root_only run?)");
+    if (E && (!g->edge_off || !g->edge_len || !g->edge_bases)) return fail(W2RAP_ERR_BAD_ARG, err, errlen, "%s", "graph without edge sequences");
+    // per hbv edge: its segment (fwd id of its canonical edge), orientation and endpoints
+    std::vector<int32_t> seg(nh, -1), left(nh), right(nh);
+    std::vector<uint8_t> minus(nh, 0);
+    for (uint64_t e = 0; e < E; ++e) {
+        const int32_t fw = g->fwd_xlat[e];
+        if (fw < 0 || (uint64_t)fw >= nh || g->involution[fw] < 0 || (uint64_t)g->involution[fw] >= nh)
+            return fail(W2RAP_ERR_BAD_ARG, err, errlen, "%s", "hbv edge id out of range");
+        const int32_t rv = g->involution[fw];
+        seg[fw] = fw; left[fw] = g->edge_vertices[4 * e]; right[fw] = g->edge_vertices[4 * e + 1];
+        if (rv != fw) { seg[rv] = fw; minus[rv] = 1; left[rv] = g->edge_vertices[4 * e + 2]; right[rv] = g->edge_vertices[4 * e + 3]; }
+    }
+    for (uint64_t x = 0; x < nh; ++x)
+        if (seg[x] < 0 || left[x] < 0 || (uint64_t)left[x] >= nv || right[x] < 0 || (uint64_t)right[x] >= nv)
+            return fail(W2RAP_ERR_BAD_ARG, err, errlen, "%s", "hbv edges and vertices are inconsistent");
+    File f(path, "w");
+    if (!f.f) return fail(W2RAP_ERR_IO, err, errlen, "cannot create %s", path);
+    bool ok = fputs("H\tVN:Z:1.0\n", f.f) >= 0;
+    std::string line;
+    for (uint64_t e = 0; e < E && ok; ++e) {
+        const uint32_t len = g->edge_len[e];
+        const uint8_t* p = g->edge_bases + g->edge_off[e];
+        line.assign("S\t");
+        line += std::to_string(g->fwd_xlat[e]);
+        line += '\t';
+        for (uint32_t i = 0; i < len; ++i) line += "ACGT"[(p[i >> 2] >> ((i & 3) * 2)) & 3u];
+        line += "\tLN:i:" + std::to_string(len);
+        if (edge_cov) {
+            char dp[64];
+            line += "\tKC:i:" + std::to_string(edge_cov[e].sum);
+            if (edge_cov[e].n_kmers) { snprintf(dp, sizeof dp, "\tDP:f:%.3f", (double)edge_cov[e].sum / (double)edge_cov[e].n_kmers); line += dp; }
+        }
+        line += '\n';
+        ok = f.put(line.data(), line.size());
+    }
+    // in-edges and out-edges of every vertex, in hbv id order
+    std::vector<uint64_t> in_off(nv + 1, 0), out_off(nv + 1, 0);
+    for (uint64_t x = 0; x < nh; ++x) { ++in_off[right[x] + 1]; ++out_off[left[x] + 1]; }
+    for (uint64_t v = 0; v < nv; ++v) { in_off[v + 1] += in_off[v]; out_off[v + 1] += out_off[v]; }
+    std::vector<int32_t> ins(nh), outs(nh);
+    {
+        std::vector<uint64_t> ci(in_off.begin(), in_off.end() - 1), co(out_off.begin(), out_off.end() - 1);
+        for (uint64_t x = 0; x < nh; ++x) { ins[ci[right[x]]++] = (int32_t)x; outs[co[left[x]]++] = (int32_t)x; }
+    }
+    const int32_t* inv = g->involution;
+    for (uint64_t v = 0; v < nv && ok; ++v)
+        for (uint64_t a = in_off[v]; a < in_off[v + 1] && ok; ++a)
+            for (uint64_t b = out_off[v]; b < out_off[v + 1] && ok; ++b) {
+                const int32_t x = ins[a], y = outs[b];
+                if (std::make_pair(inv[y], inv[x]) < std::make_pair(x, y)) continue;      // its complement is the one written
+                ok = fprintf(f.f, "L\t%d\t%c\t%d\t%c\t%dM\n", seg[x], minus[x] ? '-' : '+', seg[y], minus[y] ? '-' : '+', W2RAP_K - 1) > 0;
+            }
     if (!ok) return fail(W2RAP_ERR_IO, err, errlen, "short write to %s", path);
     return W2RAP_OK;
 }

@@ -1,10 +1,12 @@
-// step2_main.cc — file-level drop-in for step 2: `step2 <out_dir> <prefix> [--min_freq F[,F2,...]] [--min_qual Q] [--device D]`
+// step2_main.cc — file-level drop-in for step 2: `step2 <out_dir> <prefix> [--min_freq F[,F2,...]] [--min_qual Q] [--device D] [--gfa]`
 // reads <out_dir>/frag_reads_orig.fastb/.qualp (what `w2rap-contigger --to_step 1` leaves, w2rap-contigger.cc:315-316),
 // writes <out_dir>/<prefix>.small_K.hbv, .small_K.paths (post-FixPaths) and small_K.freqs, after which
 // `w2rap-contigger -o <out_dir> -p <prefix> --from_step 3` continues (w2rap-contigger.cc:352-358).
 // With a list of min_freq values the reads are read, uploaded and counted once (keep floor = the smallest value,
 // include/w2rap_step2_counts.h), small_K.freqs is written once, and every value F gets its own graph and paths,
 // <prefix>_mf<F>.small_K.hbv / .small_K.paths, continued by `w2rap-contigger -o <out_dir> -p <prefix>_mf<F> --from_step 3`.
+// --gfa: also the graph as GFA with per-edge k-mer coverage (include/w2rap_coverage.h) next to each .hbv, <prefix>.small_K.gfa or
+// <prefix>_mf<F>.small_K.gfa.  The counts must stay resident for that, so even one value goes through one count and one build.
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -13,7 +15,7 @@
 #include <vector>
 
 #include "w2rap_step2.h"
-#include "w2rap_step2_counts.h"
+#include "w2rap_coverage.h"
 
 // "3,4,5" -> {3, 4, 5}; false on anything that is not a comma-separated list of integers in 1..255
 static bool parse_min_freqs(const char* s, std::vector<uint32_t>* out) {
@@ -29,8 +31,17 @@ static bool parse_min_freqs(const char* s, std::vector<uint32_t>* out) {
     return !out->empty();
 }
 
-// one count, one build per value of `freqs` (in the order given)
-static int run_sweep(const char* dir, const char* prefix, w2rap_params p, const std::vector<uint32_t>& freqs, char* err, size_t errlen) {
+// The graph as GFA, KC/DP from the coverage of its edges in the counts.
+static int write_gfa(const std::string& path, const w2rap_counts* counts, const w2rap_graph& g, char* err, size_t errlen) {
+    const w2rap_seqs edges = {g.n_edges, g.edge_bases, g.edge_off, g.edge_len};
+    std::vector<w2rap_seq_cov> cov(g.n_edges);
+    int rc = w2rap_counts_coverage(counts, &edges, cov.data(), nullptr, err, errlen);
+    if (rc == W2RAP_OK) rc = w2rap_write_gfa(path.c_str(), &g, cov.data(), err, errlen);
+    return rc;
+}
+
+// one count, one build per value of `freqs` (in the order given); `gfa`: also <base>.gfa
+static int run_sweep(const char* dir, const char* prefix, w2rap_params p, const std::vector<uint32_t>& freqs, bool gfa, char* err, size_t errlen) {
     const std::string d(dir);
     w2rap_reads r;
     int rc = w2rap_read_fastb_qualp((d + "/frag_reads_orig.fastb").c_str(), (d + "/frag_reads_orig.qualp").c_str(), &r, err, errlen);
@@ -56,9 +67,10 @@ static int run_sweep(const char* dir, const char* prefix, w2rap_params p, const 
         w2rap_graph g;
         rc = w2rap_step2_build(reads, counts, &p, &g, err, errlen);
         if (rc) break;
-        const std::string base = d + "/" + prefix + "_mf" + std::to_string(freqs[i]) + ".small_K";
+        const std::string base = d + "/" + prefix + (freqs.size() > 1 ? "_mf" + std::to_string(freqs[i]) : std::string()) + ".small_K";
         rc = w2rap_write_hbv((base + ".hbv").c_str(), &g, err, errlen);
         if (rc == W2RAP_OK) rc = w2rap_write_paths((base + ".paths").c_str(), &g, err, errlen);
+        if (rc == W2RAP_OK && gfa) rc = write_gfa(base + ".gfa", counts, g, err, errlen);
         if (rc == W2RAP_OK) printf("TIME, build min_freq %u +FixPaths (B200), %.3f\n", freqs[i], g.timings.total_ms * 1e-3);
         w2rap_step2_free(&g);
     }
@@ -68,11 +80,12 @@ static int run_sweep(const char* dir, const char* prefix, w2rap_params p, const 
 }
 
 int main(int argc, char** argv) {
-    if (argc < 3) { fprintf(stderr, "usage: %s <out_dir> <prefix> [--min_freq F[,F2,...]] [--min_qual Q] [--device D] [--quiet]\n", argv[0]); return 2; }
+    if (argc < 3) { fprintf(stderr, "usage: %s <out_dir> <prefix> [--min_freq F[,F2,...]] [--min_qual Q] [--device D] [--gfa] [--quiet]\n", argv[0]); return 2; }
     w2rap_params p;
     memset(&p, 0, sizeof p);
     p.abi_version = W2RAP_STEP2_ABI_VERSION; p.K = W2RAP_K; p.min_qual = 7; p.min_freq = 4; p.device = -1; p.verbose = 1;
     std::vector<uint32_t> freqs = {4};
+    bool gfa = false;
     for (int i = 3; i < argc; ++i) {
         if (!strcmp(argv[i], "--min_freq") && i + 1 < argc) {
             ++i;
@@ -81,12 +94,13 @@ int main(int argc, char** argv) {
         }
         else if (!strcmp(argv[i], "--min_qual") && i + 1 < argc) p.min_qual = (uint32_t)atoi(argv[++i]);
         else if (!strcmp(argv[i], "--device") && i + 1 < argc) p.device = atoi(argv[++i]);
+        else if (!strcmp(argv[i], "--gfa")) gfa = true;
         else if (!strcmp(argv[i], "--quiet")) p.verbose = 0;
         else { fprintf(stderr, "unknown argument %s\n", argv[i]); return 2; }
     }
     char err[1024] = {0};
-    if (freqs.size() > 1) {
-        int rc = run_sweep(argv[1], argv[2], p, freqs, err, sizeof err);
+    if (freqs.size() > 1 || gfa) {
+        int rc = run_sweep(argv[1], argv[2], p, freqs, gfa, err, sizeof err);
         if (rc) { fprintf(stderr, "step2 failed (%d): %s\n", rc, err); return 1; }
         return 0;
     }
