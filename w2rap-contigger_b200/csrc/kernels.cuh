@@ -153,11 +153,12 @@ __global__ void k_adjacency(SolidTable st) {
         if (c2 != c) s->ctx = c2;     // other threads only test membership (keys), never contexts, during this kernel
     }
 }
-// The same over the dense nodes (one GPU): a sequential sweep; the neighbours are probed in the table.
+// The same over the dense nodes (one GPU): a sequential sweep; a neighbour is looked for next to its node first (unipath.cuh: node_find),
+// then probed in the table.  Other threads only read the keys of entries here, never their contexts.
 __global__ void k_adjacency_dense(DenseNodes d) {
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < d.n; i += (uint64_t)gridDim.x * blockDim.x) {
         SolidSlot* s = d.nodes + i;
-        const uint32_t c = s->ctx & 0xffu, c2 = pruned_context(d.t, Kmer{s->w0, s->w1}, c);
+        const uint32_t c = s->ctx & 0xffu, c2 = pruned_context(d, i, Kmer{s->w0, s->w1}, c);
         if (c2 != c) s->ctx = c2;
     }
 }

@@ -27,6 +27,11 @@ W2R_HD bool slot_is_ghost(const SolidSlot& s) { return s.pad != 0; }      // pad
 //   DenseNodes : id = index in the dense array of solid k-mers, in the order the reduce emitted them: grouped by minimiser and
 //                sorted by the minimiser's place (count_part.cuh), so the k-mers of a chain mostly get neighbouring ids and a chain
 //                step stays inside a sector or two.  The table's `off` field holds every key's id until the graph stage ends.
+// node_find(view, canonical k-mer, hint) -> id or -1.  `hint` is the id of the node asking.  DenseNodes first compares the keys within
+// NODE_WINDOW ids of it, nearest first: a neighbour along a chain mostly sits there, in lines the warp has just read, and only a miss
+// pays the dependent probe chain in the table plus the read of the slot's `off`.  A window hit is a full key comparison, so the answer
+// is the same in any id order.  SolidTable ignores the hint (its ids are hash-placed slots).
+constexpr int NODE_WINDOW = 4;
 struct DenseNodes {
     SolidTable t;
     SolidSlot* nodes;
@@ -35,8 +40,28 @@ struct DenseNodes {
 };
 W2R_HD SolidSlot& node_entry(const SolidTable& t, uint64_t id) { return t.slots[id]; }
 W2R_HD SolidSlot& node_entry(const DenseNodes& d, uint64_t id) { return d.nodes[id]; }
-W2R_HD int64_t node_find(const SolidTable& t, Kmer k) { return solid_find(t, k); }
-W2R_HD int64_t node_find(const DenseNodes& d, Kmer k) {
+W2R_HD int64_t node_find(const SolidTable& t, Kmer k, uint64_t) { return solid_find(t, k); }
+W2R_HD bool node_key_is(const DenseNodes& d, uint64_t j, Kmer k) {
+#if defined(__CUDA_ARCH__)
+    const ulonglong2 kk = __ldg(reinterpret_cast<const ulonglong2*>(d.nodes + j));
+    return kk.x == k.w0 && kk.y == k.w1;
+#else
+    return d.nodes[j].w0 == k.w0 && d.nodes[j].w1 == k.w1;
+#endif
+}
+// The window part alone: id of k within NODE_WINDOW ids of hint (hint itself included: a k-mer can be its own neighbour), or -1.
+W2R_HD int64_t node_find_near(const DenseNodes& d, Kmer k, uint64_t hint) {
+    if (node_key_is(d, hint, k)) return (int64_t)hint;
+#pragma unroll
+    for (int r = 1; r <= NODE_WINDOW; ++r) {
+        if (hint + r < d.n && node_key_is(d, hint + r, k)) return (int64_t)(hint + r);
+        if (hint >= (uint64_t)r && node_key_is(d, hint - r, k)) return (int64_t)(hint - r);
+    }
+    return -1;
+}
+W2R_HD int64_t node_find(const DenseNodes& d, Kmer k, uint64_t hint) {
+    const int64_t j = node_find_near(d, k, hint);
+    if (j >= 0) return j;
     const int64_t s = solid_find(d.t, k);
     return s < 0 ? -1 : (int64_t)d.t.slots[s].off;
 }
@@ -68,7 +93,7 @@ W2R_HD uint32_t unipath_succ_link(const V& t, uint32_t x, int* missing, bool* to
     Kmer nrc = kmer_rc(n);
     if (nrc == n) return NIL;                                   // :239
     bool rev = kmer_less(nrc, n);
-    int64_t ts = node_find(t, rev ? nrc : n);
+    int64_t ts = node_find(t, rev ? nrc : n, x >> 1);
     if (ts < 0) { if (missing) *missing = 1; return NIL; }
     uint32_t c2 = node_entry(t, ts).ctx & 0xffu;
     if (rev) c2 = ctx_rc(c2);
@@ -78,13 +103,21 @@ W2R_HD uint32_t unipath_succ_link(const V& t, uint32_t x, int* missing, bool* to
 }
 
 // kmers/ReadPather.h:317-346 AdjProc for one entry: clear every context bit whose neighbour k-mer is not in the dictionary.
-W2R_HD uint32_t pruned_context(const SolidTable& t, Kmer k, uint32_t c) {
+// id = the entry's node id (the hint of node_find).
+template <class V>
+W2R_HD bool node_has(const V& v, Kmer k, uint64_t id) {
+    const Kmer r = kmer_rc(k);
+    return node_find(v, kmer_less(r, k) ? r : k, id) >= 0;
+}
+template <class V>
+W2R_HD uint32_t pruned_context(const V& v, uint64_t id, Kmer k, uint32_t c) {
     for (uint32_t b = 0; b < 4; ++b)
-        if (c & (1u << b)) { if (solid_find_any(t, kmer_succ(k, b), nullptr) < 0) c &= ~(1u << b); }
+        if (c & (1u << b)) { if (!node_has(v, kmer_succ(k, b), id)) c &= ~(1u << b); }
     for (uint32_t b = 0; b < 4; ++b)
-        if (c & (16u << b)) { if (solid_find_any(t, kmer_pred(k, b), nullptr) < 0) c &= ~(16u << b); }
+        if (c & (16u << b)) { if (!node_has(v, kmer_pred(k, b), id)) c &= ~(16u << b); }
     return c;
 }
+W2R_HD uint32_t pruned_context(const SolidTable& t, Kmer k, uint32_t c) { return pruned_context(t, 0, k, c); }
 
 
 // ---------------------------------------------------------------- list ranking by pointer jumping
