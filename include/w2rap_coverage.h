@@ -7,7 +7,8 @@
  * every 60-mer seen at least f0 times, so the coverage of the graph's edges (or of reads, or of contigs) is a lookup of every
  * k-mer of a sequence in those counts.
  *
- * Single GPU, on the device the counts live on.  Exported from libw2rap_step2.so, next to w2rap_step2.h.
+ * Single GPU, on the device the counts live on; for sharded counts see w2rap_counts_coverage_sharded (w2rap_step2_counts_sharded.h).
+ * Exported from libw2rap_step2.so, next to w2rap_step2.h.
  *
  *   w2rap_step2_count(reads, &p, &counts, NULL, err, n);               p.min_freq = f0
  *   w2rap_step2_build(reads, counts, &p, &g, err, n);                  p.min_freq = F >= f0

@@ -9,7 +9,8 @@
  * paths (+FixPaths) and places.  Its result is identical, in every field except the timings, to w2rap_step2_run_resident() on
  * the same reads with the same min_qual and min_freq.
  *
- * Single GPU only (no communicator).  Exported from libw2rap_step2.so, next to w2rap_step2.h.
+ * Single GPU (no communicator); the sharded forms are in w2rap_step2_counts_sharded.h.  Exported from libw2rap_step2.so, next to
+ * w2rap_step2.h.
  *
  *   w2rap_device_reads* reads;  w2rap_step2_upload(&host_reads, device, &reads, err, n);
  *   w2rap_counts* counts;       p.min_freq = 3;  w2rap_step2_count(reads, &p, &counts, &spectrum, err, n);

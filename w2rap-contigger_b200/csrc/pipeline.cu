@@ -41,8 +41,11 @@ struct w2rap_counts {
     uint64_t n_reads = 0, n_bases = 0;              // ... still holding the same reads
     int device = 0;
     uint32_t min_qual = 0, f0 = 0;                  // quality floor of the count; keep floor (every k-mer seen >= f0 times is kept)
-    uint64_t n_kmer_instances = 0, n_distinct = 0, n_kept = 0;
-    uint64_t hist[101] = {};
+    uint64_t n_kmer_instances = 0, n_distinct = 0, n_kept = 0;     // n_kept: on this rank
+    uint64_t hist[101] = {};                        // (whole-job counters: identical on every rank of a sharded count)
+    const w2rap_comm* comm = nullptr;               // sharded count: the communicator (null: single GPU), this rank, the world ...
+    int world = 1, rank = 0;
+    uint32_t logP = 0;                              // ... and the partition count 2^logP: a k-mer is kept on its partition's owner
     ulonglong2* solid = nullptr;                    // n_kept records {w0, w1 | raw ctx}, in the order the reduce emitted them
     uint8_t* count = nullptr;                       // n_kept counts, min(255, occurrences), parallel to `solid`
 };
@@ -843,6 +846,7 @@ struct Pipeline {
         out->n_kmer_instances = h.n_kmer_instances;
         for (int i = 0; i <= 100; ++i) out->hist[i] = h.hist[i];
         n_distinct_ = h.n_distinct;
+        count_logP_ = h.logP;                   // sharded: the graph stage finds a k-mer's owner by the count's partition layout
         n_solid_local_ = 0;
         cs_solid.alloc(c, h.n_kept);
         if (!h.n_kept) return;
@@ -1711,8 +1715,10 @@ struct Pipeline {
         say(c, "creating kmers from reads...");
         count_stage();
         const uint64_t n = n_solid_local_;
-        out->n_distinct = n_distinct_; out->n_solid = n;
-        say(c, "%llu kmers counted, %llu with Freq >= %u kept", (unsigned long long)n_distinct_, (unsigned long long)n, prm.min_freq);
+        std::vector<unsigned long long> kept = {n};
+        allreduce_u64(kept, ncclSum);              // sharded: the summary counts what all ranks keep
+        out->n_distinct = n_distinct_; out->n_solid = kept[0];
+        say(c, "%llu kmers counted, %llu with Freq >= %u kept", (unsigned long long)n_distinct_, kept[0], prm.min_freq);
         const double t0 = now_ms();
         cudaError_t e = cudaMallocAsync((void**)&h->solid, std::max<uint64_t>(n, 1) * sizeof(ulonglong2), c.stream);
         if (e == cudaSuccess) e = cudaMallocAsync((void**)&h->count, std::max<uint64_t>(n, 1), c.stream);
@@ -1724,7 +1730,7 @@ struct Pipeline {
         }
         W2R_CUDA(cudaStreamSynchronize(c.stream));
         cs_solid.release(); cs_count.release(); good.release();
-        h->n_kept = n; h->n_distinct = n_distinct_; h->n_kmer_instances = out->n_kmer_instances;
+        h->n_kept = n; h->n_distinct = n_distinct_; h->n_kmer_instances = out->n_kmer_instances; h->logP = count_logP_;
         for (int i = 0; i <= 100; ++i) h->hist[i] = out->hist[i];
         if (!dump_host.empty()) {
             std::sort(dump_host.begin(), dump_host.end(), [](const DumpRec& a, const DumpRec& b) { return a.w0 < b.w0 || (a.w0 == b.w0 && a.w1 < b.w1); });
@@ -1926,6 +1932,63 @@ static void run_on_device(DeviceReads& dr, const w2rap_params* p, w2rap_graph* o
     }
 }
 
+// Which calls a counts handle may go to: a sharded count only to the sharded calls with its own communicator (every rank holds
+// only its partitions), a single-GPU count only to the single-GPU calls.  Shared by every entry point that takes a handle.
+static void check_counts_comm(const w2rap_counts* h, const w2rap_comm* comm) {
+    if (h->comm && !comm) W2R_FAIL(W2RAP_ERR_BAD_ARG, "these counts are sharded (w2rap_step2_count_sharded): they hold this rank's partitions only; use the _sharded calls");
+    if (!h->comm && comm) W2R_FAIL(W2RAP_ERR_BAD_ARG, "these counts were made on one GPU (w2rap_step2_count): use the single-GPU calls");
+    if (h->comm != comm) W2R_FAIL(W2RAP_ERR_BAD_ARG, "these counts were made with another communicator: use the one they were counted with");
+}
+
+// The argument checks of a count, on one GPU (sharded = false, comm unused) or sharded.  Made before any device work or collective.
+static void check_count_args(const w2rap_device_reads* reads, const w2rap_params* p, w2rap_counts** counts, const w2rap_comm* comm, bool sharded) {
+    if (!reads || !counts || (sharded && !comm)) W2R_FAIL(W2RAP_ERR_BAD_ARG, "null argument");
+    *counts = nullptr;
+    check_params(p);
+    if (sharded && p->dump_kmers) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers must be 0 for a sharded count (level 2 is a single-GPU test hook, level 1 dumps the dictionary of a build)");
+    if (p->dump_kmers == 1) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers 1 dumps the solid dictionary, which only a build makes: a count takes dump_kmers 0 or 2");
+    if (p->dump_kmers > 2) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers must be 0 or 2 for a count");
+    if (sharded && reads->d.device != comm->device) W2R_FAIL(W2RAP_ERR_BAD_ARG, "read shard lives on device %d, communicator on %d", reads->d.device, comm->device);
+}
+
+// The argument checks of a build, on one GPU (comm = null) or sharded.  Made before any device work or collective.
+static void check_build_args(const w2rap_device_reads* reads, const w2rap_counts* counts, const w2rap_params* p, const w2rap_graph* out, const w2rap_comm* comm,
+                             bool sharded) {
+    if (!reads || !counts || !out || (sharded && !comm)) W2R_FAIL(W2RAP_ERR_BAD_ARG, "null argument");
+    check_params(p);
+    check_counts_comm(counts, comm);
+    if (p->min_freq < counts->f0)
+        W2R_FAIL(W2RAP_ERR_BAD_ARG, "min_freq %u is below the keep floor %u of these counts (k-mers seen fewer times were not kept): count again with min_freq <= %u",
+                 p->min_freq, counts->f0, p->min_freq);
+    if (p->min_qual != counts->min_qual)
+        W2R_FAIL(W2RAP_ERR_BAD_ARG, "min_qual %u differs from the min_qual %u these counts were made with (the quality floor changes the counts): count again",
+                 p->min_qual, counts->min_qual);
+    if (p->dump_kmers == 2) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers 2 (every distinct k-mer with its count) comes from w2rap_step2_count, not from a build");
+    if (p->dump_kmers > 2) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers must be 0 or 1 for a build");
+    if (reads != counts->reads || reads->d.n != counts->n_reads || reads->d.n_bases != counts->n_bases)
+        W2R_FAIL(W2RAP_ERR_BAD_ARG, "the reads handle is not the one these counts were made from: a build paths the reads that were counted");
+}
+
+// w2rap_step2_count(_sharded) after the checks: the count stage into a new handle, and <workdir>/small_K.freqs from rank 0.
+static int count_into_handle(w2rap_device_reads* reads, const w2rap_params* p, const w2rap_comm* comm, w2rap_counts** counts, w2rap_graph* summary,
+                             char* err, size_t errlen) {
+    w2rap_counts* h = new w2rap_counts();
+    h->reads = reads; h->n_reads = reads->d.n; h->n_bases = reads->d.n_bases; h->device = reads->d.device;
+    h->min_qual = p->min_qual; h->f0 = p->min_freq;
+    if (comm) { h->comm = comm; h->world = comm->world; h->rank = comm->rank; }
+    w2rap_graph local;
+    w2rap_graph* out = summary ? summary : &local;
+    try {
+        run_on_device(reads->d, p, out, 0.f, comm, 0, h);
+    } catch (...) { w2rap_step2_counts_release(h); throw; }
+    int rc = W2RAP_OK;
+    if (h->rank == 0 && p->workdir && p->workdir[0]) { std::string f = std::string(p->workdir) + "/small_K.freqs"; rc = w2rap_write_freqs(f.c_str(), out, err, errlen); }
+    if (!summary) w2rap_step2_free(&local);
+    if (rc) { w2rap_step2_counts_release(h); return rc; }
+    *counts = h;
+    return W2RAP_OK;
+}
+
 }  // namespace w2r
 
 // ================================================================ C ABI
@@ -2082,46 +2145,34 @@ int w2rap_step2_run_sharded(const w2rap_reads* shard, const w2rap_params* p, w2r
     W2R_API_END
 }
 
-// ---- count once, build for several min_freq (include/w2rap_step2_counts.h)
+// ---- count once, build for several min_freq (include/w2rap_step2_counts.h, include/w2rap_step2_counts_sharded.h)
 int w2rap_step2_count(w2rap_device_reads* reads, const w2rap_params* p, w2rap_counts** counts, w2rap_graph* summary, char* err, size_t errlen) {
     W2R_API_BEGIN
-    if (!reads || !counts) W2R_FAIL(W2RAP_ERR_BAD_ARG, "null argument");
-    *counts = nullptr;
-    check_params(p);
-    if (p->dump_kmers == 1) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers 1 dumps the solid dictionary, which only a build makes: a count takes dump_kmers 0 or 2");
-    if (p->dump_kmers > 2) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers must be 0 or 2 for a count");
-    w2rap_counts* h = new w2rap_counts();
-    h->reads = reads; h->n_reads = reads->d.n; h->n_bases = reads->d.n_bases; h->device = reads->d.device;
-    h->min_qual = p->min_qual; h->f0 = p->min_freq;
-    w2rap_graph local;
-    w2rap_graph* out = summary ? summary : &local;
-    try {
-        run_on_device(reads->d, p, out, 0.f, nullptr, 0, h);
-    } catch (...) { w2rap_step2_counts_release(h); throw; }
-    int rc = W2RAP_OK;
-    if (p->workdir && p->workdir[0]) { std::string f = std::string(p->workdir) + "/small_K.freqs"; rc = w2rap_write_freqs(f.c_str(), out, err, errlen); }
-    if (!summary) w2rap_step2_free(&local);
-    if (rc) { w2rap_step2_counts_release(h); return rc; }
-    *counts = h;
+    check_count_args(reads, p, counts, nullptr, false);
+    if (int rc = count_into_handle(reads, p, nullptr, counts, summary, err, errlen)) return rc;
+    W2R_API_END
+}
+
+int w2rap_step2_count_sharded(w2rap_device_reads* shard, const w2rap_params* p, w2rap_comm* comm, w2rap_counts** counts, w2rap_graph* summary, char* err, size_t errlen) {
+    W2R_API_BEGIN
+    check_count_args(shard, p, counts, comm, true);
+    if (int rc = count_into_handle(shard, p, comm, counts, summary, err, errlen)) return rc;
     W2R_API_END
 }
 
 int w2rap_step2_build(w2rap_device_reads* reads, const w2rap_counts* counts, const w2rap_params* p, w2rap_graph* out, char* err, size_t errlen) {
     W2R_API_BEGIN
-    if (!reads || !counts || !out) W2R_FAIL(W2RAP_ERR_BAD_ARG, "null argument");
-    check_params(p);
-    if (p->min_freq < counts->f0)
-        W2R_FAIL(W2RAP_ERR_BAD_ARG, "min_freq %u is below the keep floor %u of these counts (k-mers seen fewer times were not kept): count again with min_freq <= %u",
-                 p->min_freq, counts->f0, p->min_freq);
-    if (p->min_qual != counts->min_qual)
-        W2R_FAIL(W2RAP_ERR_BAD_ARG, "min_qual %u differs from the min_qual %u these counts were made with (the quality floor changes the counts): count again",
-                 p->min_qual, counts->min_qual);
-    if (p->dump_kmers == 2) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers 2 (every distinct k-mer with its count) comes from w2rap_step2_count, not from a build");
-    if (p->dump_kmers > 2) W2R_FAIL(W2RAP_ERR_BAD_ARG, "dump_kmers must be 0 or 1 for a build");
-    if (reads != counts->reads || reads->d.n != counts->n_reads || reads->d.n_bases != counts->n_bases)
-        W2R_FAIL(W2RAP_ERR_BAD_ARG, "the reads handle is not the one these counts were made from: a build paths the reads that were counted");
+    check_build_args(reads, counts, p, out, nullptr, false);
     run_on_device(reads->d, p, out, 0.f, nullptr, 0, nullptr, counts);
     if (p->workdir && p->workdir[0]) { std::string f = std::string(p->workdir) + "/small_K.freqs"; int rc = w2rap_write_freqs(f.c_str(), out, err, errlen); if (rc) return rc; }
+    W2R_API_END
+}
+
+int w2rap_step2_build_sharded(w2rap_device_reads* shard, const w2rap_counts* counts, const w2rap_params* p, w2rap_comm* comm, w2rap_graph* out, char* err, size_t errlen) {
+    W2R_API_BEGIN
+    check_build_args(shard, counts, p, out, comm, true);
+    run_on_device(shard->d, p, out, 0.f, comm, 0, nullptr, counts);
+    if (comm->rank == 0 && p->workdir && p->workdir[0]) { std::string f = std::string(p->workdir) + "/small_K.freqs"; int rc = w2rap_write_freqs(f.c_str(), out, err, errlen); if (rc) return rc; }
     W2R_API_END
 }
 
